@@ -69,6 +69,9 @@ def parse():
                          "multi-view file driver (C3, C4 = 300 views); auto: driver for C3 / C4, engine otherwise")
     ap.add_argument("--lanes", type=int, default=2, help="pipelined contexts per GPU of the multi-view driver (--config C3 / C4)")
     ap.add_argument("--io_threads", type=int, default=6, help="decoder / writer threads per rank of the multi-view driver")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps write what the last timed step computed as DIR/<name>.npy (per-view path, "
+                         "rank 0): depth, normals and confidence at a fixed sample of pixels, and the superpixel labels")
     return ap.parse_args()
 
 
@@ -217,6 +220,20 @@ def cpu_baseline(pkg, cfg, evals_per_depthmap):
             "host_cores_available": os.cpu_count()}
 
 
+def dump_outputs(out_dir, norm4, confid, labels, n_sample=1 << 20):
+    """What a caller of the per-view path receives, as float32 / float64 .npy files (31 MB at C2): depth, normals and
+    confidence at n_sample pixels drawn with a fixed seed (the full C2 maps would be 127 MB), and the superpixel labels
+    in full."""
+    os.makedirs(out_dir, exist_ok=True)
+    H, W = confid.shape
+    idx = np.sort(np.random.RandomState(0).choice(H * W, min(n_sample, H * W), replace=False))
+    n4 = norm4.reshape(H * W, 4)[idx]
+    arrays = {"pixel_index": idx.astype(np.float64), "depth": n4[:, 3], "normals": n4[:, :3], "confidence": confid.reshape(-1)[idx],
+              "superpixel_labels": labels.astype(np.float64)}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.ascontiguousarray(a))
+
+
 def run_ours(args):
     import torch
     import __graft_entry__ as g
@@ -242,11 +259,12 @@ def run_ours(args):
     eng.upload(L.F_CANNY, canny)            # region labels of the reference view (caller input, resident)
 
     def step_resident(seed):
-        eng.slic(bgrx)                      # quarter-resolution colour image of the reference view
+        labels = eng.slic(bgrx)             # quarter-resolution colour image of the reference view
         eng.init_planes(seed)
         eng.iterate(iters, seed)
         eng.lrdiff(); eng.getview()
         eng.update_scale_2(); eng.update_scale(); eng.compute_disp()
+        return labels
 
     n_evals = eng.eval_count(iters)
     for _ in range(args.warmup):
@@ -264,9 +282,11 @@ def run_ours(args):
             if flush is not None:
                 flush.fill_(k)
             evs[k][0].record()
-            step_resident(SEED + 100 * k)
+            labels = step_resident(SEED + 100 * k)
             evs[k][1].record()
         torch.cuda.synchronize()
+    if args.dump_outputs and rank == 0 and args.steps > 0:
+        dump_outputs(args.dump_outputs, eng.download(L.F_NORM4), eng.download(L.F_CONFID), labels)
     ms_local = sum(a.elapsed_time(b) for a, b in evs)
     barrier(world)
     ms = max_over_ranks(ms_local, world)
@@ -567,6 +587,8 @@ if __name__ == "__main__":
     driver = a.config in PRODUCT_CONFIGS and a.mode != "engine"
     if a.mode == "driver" and a.config not in PRODUCT_CONFIGS:
         sys.exit(f"--mode driver needs one of {sorted(PRODUCT_CONFIGS)}")
+    if a.dump_outputs and (a.impl == "reference" or driver):
+        sys.exit("--dump-outputs writes the outputs of the per-view path (--impl ours, per-view configs or --mode engine)")
     if a.impl == "reference" and driver:
         if int(os.environ.get("RANK", "0")) == 0:
             emit({"impl": "reference", "unavailable": "the reference has no multi-view driver (one process per view, scripts/pipes.sh); "

@@ -141,3 +141,21 @@ def ref_slic(bgrx, spixel_size=20, no_iters=5, coh_weight=5.0, enforce_connectiv
     if rc != 0:
         raise RuntimeError(f"ref_slic failed ({rc})")
     return labels, ms.value
+
+
+def slic_last_lab(n):
+    """CIELab image [n][4] of the last ref_slic call (the reference engine's own buffer)."""
+    lib = C.CDLL(os.path.join(REF_DIR, "libgslic_ref.so"))
+    lib.ref_slic_last_lab.restype = C.c_longlong
+    lib.ref_slic_last_lab.argtypes = [C.c_void_p, C.c_longlong]
+    out = np.empty((n, 4), np.float32)
+    lib.ref_slic_last_lab(out.ctypes.data, n)
+    return out
+
+
+def slic_last_centres(nsp):
+    """Superpixel records [nsp][8] (centre, colour, count) of the last ref_slic call."""
+    lib = C.CDLL(os.path.join(REF_DIR, "libgslic_ref.so"))
+    out = np.zeros((nsp, 8), np.float32)
+    lib.ref_slic_last_centres(out.ctypes.data_as(C.c_void_p), nsp)
+    return out

@@ -25,13 +25,42 @@ def load_pkg():
 
 
 def ref_binding():
-    from oracle import ref_binding as rb
-    return rb
+    """The reference's own kernels (oracle/_ref, built by `make oracle` where the reference checkout exists), else their
+    recorded results (oracle/recorded.py).  With TSAR_RECORD_REFERENCE_DIGESTS set, the reference build's results are
+    recorded; that needs the build."""
+    from oracle import recorded, ref_binding as rb
+    built = all(rb.available(v) for v in ("asis", "snapshot", "snapshot_init")) and os.path.exists(os.path.join(rb.REF_DIR, "libgslic_ref.so"))
+    if os.environ.get("TSAR_RECORD_REFERENCE_DIGESTS"):
+        assert built, "recording reference results needs the reference build (oracle/_ref: `make oracle` with the reference checkout)"
+        return recorded.recording()
+    return rb if built else recorded
 
 
-def make_engines(pkg, scene, box=11, iterations=8, n_best=1, cost_comb=1, variants=("asis",), device=0, color_processing=0):
+def ref_host():
+    """The reference's own host code (oracle/_ref/libtsar_ref_host.so), else its recorded results."""
+    from oracle import recorded, ref_host_binding as rh
+    if os.environ.get("TSAR_RECORD_REFERENCE_DIGESTS"):
+        assert rh.available(), "recording reference results needs the reference build (oracle/_ref/libtsar_ref_host.so)"
+        return recorded.recording_host()
+    return rh if rh.available() else recorded.host
+
+
+def record(name, obj):
+    """Writes a JSON record of a sweep or a full-size comparison into $TSAR_RECORD_DIR (default: a directory of the user's
+    under the system's temporary directory); returns its path."""
+    import json
+    import tempfile
+    out = os.environ.get("TSAR_RECORD_DIR") or os.path.join(tempfile.gettempdir(), f"tsar-mvs_b200-records-{os.getuid()}")
+    os.makedirs(out, exist_ok=True)
+    path = os.path.join(out, name)
+    with open(path, "w") as f:
+        json.dump(obj, f, indent=1)
+    return path
+
+
+def make_engines(pkg, scene, box=11, iterations=8, n_best=1, cost_comb=1, variants=("asis",), device=0, color_processing=0, rb=None):
     """Returns (params, mine, {variant: RefEngine}) on the same scene."""
-    rb = ref_binding()
+    rb = rb or ref_binding()
     params = pkg.make_params(box=box, iterations=iterations, n_best=n_best, cost_comb=cost_comb,
                              min_disparity=scene["min_disparity"], max_disparity=scene["max_disparity"],
                              color_processing=color_processing)
@@ -111,9 +140,9 @@ def run_smoke_check(pkg):
     """One tiny depthmap through the C ABI on cuda:0, checked against the reference-kernel oracle when it
     travelled with the repo (oracle/_ref), else against the committed golden output."""
     scene = pkg.scene.make_scene("tiny")
-    rb = ref_binding()
+    from oracle import ref_binding as rb
     variants = ("snapshot",) if rb.available("snapshot") else ()
-    params, mine, refs = make_engines(pkg, scene, iterations=2, variants=variants)
+    params, mine, refs = make_engines(pkg, scene, iterations=2, variants=variants, rb=rb)
     xy, planes = random_planes(scene, 2000)
     c_m, b_m, r_m = mine.eval_planes(xy, planes, wrapper_rounding=True)
     ms = mine.depthmap(20240601)

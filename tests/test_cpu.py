@@ -262,35 +262,78 @@ def test_bench_reference_arm_contract():
     assert "DepthmapEngine" not in ref_arm and "_lib.load" not in ref_arm   # the product library stays out of the reference arm
 
 
-def test_abi_layout_matches_reference(tmp_path):
-    """include/tsar_gipuma_abi.h against the reference's own headers: every field offset and size, compiled side by
-    side (only where the reference checkout exists; the GPU box does not have it)."""
-    ref = os.environ.get("TSAR_REFERENCE_DIR", "/root/reference")
-    if not os.path.exists(os.path.join(ref, "globalstate.h")):
-        pytest.skip("reference checkout not present")
-    fields = {
-        "Camera_cu": "P P_col34 P_inv M_inv R R_orig R_orig_inv t4 C4 fx fy f alpha baseline reference depthMin depthMax id K K_inv",
-        "CameraParameters_cu": "f rectified cameras idRef cols rows viewSelectionSubset viewSelectionSubsetNumber",
-        "LineState": "norm4 c depth fakedepth resize4 canny cenxi cenyi nein neip nump eacp ranp pind borlen depdif scale ransa "
-                     "text XYZ ratio beview lrdiff confid ranumax size n s l",
-        "AlgorithmParameters": "algorithm max_disparity min_disparity box_hsize box_vsize tau_color tau_gradient alpha gamma "
-                               "border_value iterations color_processing dispTol normTol census_epsilon self_similarity_n cam_scale "
-                               "num_img_processed costThresh good_factor n_best cost_comb viewSelection depthMin depthMax min_angle "
-                               "max_angle no_texture_sim no_texture_per max_views cols rows thres",
-        "GlobalState": "cameras lines cannylines cs params col row imgs cuArray",
-    }
-    src = ['#include "globalstate.h"', '#include "tsar_gipuma_abi.h"', "#include <cstddef>"]
-    for t, fs in fields.items():
-        src.append(f'static_assert(sizeof(::{t}) == sizeof(tsar_abi::{t}), "sizeof {t}");')
-        src.append(f'static_assert(alignof(::{t}) == alignof(tsar_abi::{t}), "alignof {t}");')
-        for f in fs.split():
-            src.append(f'static_assert(offsetof(::{t}, {f}) == offsetof(tsar_abi::{t}, {f}), "{t}::{f}");')
+# Layouts of the reference's types that include/tsar_gipuma_abi.h and include/tsar_gslicr_abi.h mirror: per type, the mirror's
+# name and {reference member: mirror member}.  tests/golden/abi_layout.json stores sizeof, alignof and every offsetof as the
+# reference's headers give them; the mirrors are compiled alone against those numbers, and the reference's headers are
+# compiled against them too where a checkout of the reference is named by TSAR_REFERENCE_DIR.
+GIPUMA_ABI_FIELDS = {
+    "Camera_cu": "P P_col34 P_inv M_inv R R_orig R_orig_inv t4 C4 fx fy f alpha baseline reference depthMin depthMax id K K_inv",
+    "CameraParameters_cu": "f rectified cameras idRef cols rows viewSelectionSubset viewSelectionSubsetNumber",
+    "LineState": "norm4 c depth fakedepth resize4 canny cenxi cenyi nein neip nump eacp ranp pind borlen depdif scale ransa "
+                 "text XYZ ratio beview lrdiff confid ranumax size n s l",
+    "AlgorithmParameters": "algorithm max_disparity min_disparity box_hsize box_vsize tau_color tau_gradient alpha gamma "
+                           "border_value iterations color_processing dispTol normTol census_epsilon self_similarity_n cam_scale "
+                           "num_img_processed costThresh good_factor n_best cost_comb viewSelection depthMin depthMax min_angle "
+                           "max_angle no_texture_sim no_texture_per max_views cols rows thres",
+    "GlobalState": "cameras lines cannylines cs params col row imgs cuArray",
+}
+GSLICR_ABI_FIELDS = {
+    "gSLICr::objects::settings": ("tsar_gslicr_abi::SettingsMirror", {
+        "img_size": "img_w", "no_segs": "no_segs", "spixel_size": "spixel_size", "no_iters": "no_iters", "coh_weight": "coh_weight",
+        "do_enforce_connectivity": "do_enforce_connectivity", "color_space": "color_space", "seg_method": "seg_method"}),
+    "ORUtils::Image<int>": ("tsar_gslicr_abi::ImageMirror", {
+        "isAllocated_CPU": "isAllocated_CPU", "data_cpu": "data_cpu", "data_cuda": "data_cuda", "dataSize": "dataSize", "noDims": "dims_x"}),
+}
+# values of the reference's gSLICr headers the shim relies on without a mirror (the enums it reads as ints, the class size)
+GSLICR_REFERENCE_VALUES = ("sizeof(gSLICr::engines::core_engine)", "gSLICr::CIELAB", "gSLICr::GIVEN_NUM", "gSLICr::GIVEN_SIZE")
+
+
+def _abi_golden():
+    import json
+    return json.load(open(os.path.join(GOLD, "abi_layout.json")))
+
+
+def _reference_dir(probe):
+    ref = os.environ.get("TSAR_REFERENCE_DIR")
+    return ref if ref and os.path.exists(os.path.join(ref, probe)) else None
+
+
+def _layout(tmp_path, headers, include_dirs, types, values=()):
+    """Compiles and runs a host program printing {label: [sizeof, alignof, {member label: offsetof}]} for
+    types = {label: (C++ type, {member label: member})}, and {expression: value} for values."""
+    import json
+    q = '\\"'
+    out = []
+    for label, (ty, members) in types.items():
+        fmt = ", ".join(f"{q}{m}{q}: %zu" for m in members)
+        args = "".join(f", (size_t)offsetof({ty}, {m})" for m in members.values())
+        out.append(f'std::printf("{q}{label}{q}: [%zu, %zu, {{{fmt}}}], ", sizeof({ty}), alignof({ty}){args});')
+    for v in values:
+        out.append(f'std::printf("{q}{v}{q}: %zu, ", (size_t)({v}));')
+    src = "\n".join([f'#include "{h}"' for h in headers] + ["#include <cstddef>", "#include <cstdio>", "int main() {", 'std::printf("{");']
+                    + out + ['std::printf("}\\n");', "return 0;", "}"])
     cu = tmp_path / "layout.cu"
-    cu.write_text("\n".join(src) + "\nint main(){return 0;}\n")
-    r = subprocess.run(["/usr/local/cuda/bin/nvcc", "-std=c++14", "-w", "-Wno-deprecated-gpu-targets", "-c", str(cu), "-o", str(tmp_path / "l.o"),
-                        "-I", os.path.join(ROOT, "oracle", "stubs"), "-I", ref, "-I", os.path.join(ROOT, "include")],
-                       capture_output=True, text=True)
+    cu.write_text(src)
+    exe = str(tmp_path / "layout")
+    inc = sum((["-I", d] for d in include_dirs + [os.path.join(ROOT, "include")]), [])
+    r = subprocess.run(["/usr/local/cuda/bin/nvcc", "-std=c++14", "-w", "-Wno-deprecated-gpu-targets", "-Xcompiler", "-Wno-invalid-offsetof",
+                        str(cu), "-o", exe] + inc, capture_output=True, text=True)
     assert r.returncode == 0, r.stderr[-3000:]
+    text = subprocess.run([exe], capture_output=True, text=True, check=True).stdout.strip()
+    return json.loads(text[:-3] + "}" if text.endswith(", }") else text)
+
+
+def test_abi_layout_matches_reference(tmp_path):
+    """include/tsar_gipuma_abi.h against the reference's own headers (globalstate.h and what it includes): sizeof, alignof
+    and every field offset of the five types, against the stored numbers and, where the checkout exists, against the
+    headers themselves."""
+    want = _abi_golden()["gipuma"]
+    mirror = {t: (f"tsar_abi::{t}", {f: f for f in fs.split()}) for t, fs in GIPUMA_ABI_FIELDS.items()}
+    assert _layout(tmp_path, ["tsar_gipuma_abi.h"], [], mirror) == want
+    ref = _reference_dir("globalstate.h")
+    if ref:
+        theirs = {t: (f"::{t}", {f: f for f in fs.split()}) for t, fs in GIPUMA_ABI_FIELDS.items()}
+        assert _layout(tmp_path, ["globalstate.h"], [os.path.join(ROOT, "oracle", "stubs"), ref], theirs) == want
 
 
 def test_gslicr_shim_layout_matches_reference(tmp_path, pkg):
@@ -301,28 +344,16 @@ def test_gslicr_shim_layout_matches_reference(tmp_path, pkg):
                    "Process_Frame(ORUtils::Image<ORUtils::Vector4<unsigned char> >*, GlobalState*)", "Get_Seg_Res()",
                    "Draw_Segmentation_Result(ORUtils::Image<ORUtils::Vector4<unsigned char> >*)", "Write_Seg_Res_To_PGM(char const*)"):
         assert f" T gSLICr::engines::core_engine::{member}" in out, member
-    ref = os.environ.get("TSAR_REFERENCE_DIR", "/root/reference")
-    if not os.path.exists(os.path.join(ref, "gSLICr_Lib", "gSLICr.h")):
-        pytest.skip("reference checkout not present")
-    src = ['#include "gSLICr_Lib/gSLICr.h"', '#include "tsar_gslicr_abi.h"', "#include <cstddef>",
-           "typedef gSLICr::objects::settings S; typedef tsar_gslicr_abi::SettingsMirror M;",
-           "typedef ORUtils::Image<int> I; typedef tsar_gslicr_abi::ImageMirror J;",
-           'static_assert(sizeof(S) == sizeof(M), "settings size");', 'static_assert(sizeof(I) == sizeof(J), "image size");',
-           'static_assert(sizeof(gSLICr::engines::core_engine) == sizeof(void *), "core_engine holds one pointer");']
-    for a, b in (("img_size", "img_w"), ("no_segs", "no_segs"), ("spixel_size", "spixel_size"), ("no_iters", "no_iters"),
-                 ("coh_weight", "coh_weight"), ("do_enforce_connectivity", "do_enforce_connectivity"), ("color_space", "color_space"),
-                 ("seg_method", "seg_method")):
-        src.append(f'static_assert(offsetof(S, {a}) == offsetof(M, {b}), "settings::{a}");')
-    for a, b in (("isAllocated_CPU", "isAllocated_CPU"), ("data_cpu", "data_cpu"), ("data_cuda", "data_cuda"), ("dataSize", "dataSize"),
-                 ("noDims", "dims_x")):
-        src.append(f'static_assert(offsetof(I, {a}) == offsetof(J, {b}), "image::{a}");')
-    src.append('static_assert(gSLICr::CIELAB == 0 && gSLICr::GIVEN_NUM == 0 && gSLICr::GIVEN_SIZE == 1, "enums");')
-    cu = tmp_path / "layout_slic.cu"
-    cu.write_text("\n".join(src) + "\nint main(){return 0;}\n")
-    r = subprocess.run(["/usr/local/cuda/bin/nvcc", "-std=c++14", "-w", "-Wno-deprecated-gpu-targets", "-Xcompiler", "-Wno-invalid-offsetof", "-c", str(cu),
-                        "-o", str(tmp_path / "l.o"), "-I", os.path.join(ROOT, "oracle", "stubs"), "-I", ref, "-I", os.path.join(ROOT, "include")],
-                       capture_output=True, text=True)
-    assert r.returncode == 0, r.stderr[-3000:]
+    golden = _abi_golden()
+    mirror = {t: (m, {a: b for a, b in fields.items()}) for t, (m, fields) in GSLICR_ABI_FIELDS.items()}
+    assert _layout(tmp_path, ["tsar_gslicr_abi.h"], [], mirror) == golden["gslicr"]
+    assert golden["gslicr_reference_values"]["sizeof(gSLICr::engines::core_engine)"] == C.sizeof(C.c_void_p)   # one pointer
+    ref = _reference_dir(os.path.join("gSLICr_Lib", "gSLICr.h"))
+    if ref:
+        theirs = {t: (t, {a: a for a in fields}) for t, (_, fields) in GSLICR_ABI_FIELDS.items()}
+        got = _layout(tmp_path, ["gSLICr_Lib/gSLICr.h"], [os.path.join(ROOT, "oracle", "stubs"), ref], theirs, GSLICR_REFERENCE_VALUES)
+        assert {t: got[t] for t in theirs} == golden["gslicr"]
+        assert {v: got[v] for v in GSLICR_REFERENCE_VALUES} == golden["gslicr_reference_values"]
 
 
 def test_cli_flag_parsing_matches_run_scripts(pkg):
@@ -438,12 +469,9 @@ def test_weak_texture_detector_finds_the_textureless_facet(pkg):
 
 
 # ---- rows f1 / f3 pinned to the reference's OWN host code (oracle/_ref/libtsar_ref_host.so = main.cpp line ranges compiled by
-# oracle/build_ref.sh; OpenCV library calls served by cv2) --------------------------------------------------------------
+# oracle/build_ref.sh; OpenCV library calls served by cv2), or to its recorded results where that build is absent -------
 def _ref_host():
-    from oracle import ref_host_binding as rh
-    if not rh.available():
-        pytest.fail("oracle/_ref/libtsar_ref_host.so missing: run `make oracle` where the reference checkout exists")
-    return rh
+    return pc.ref_host()
 
 
 def test_weak_texture_stages_match_reference_code(pkg):

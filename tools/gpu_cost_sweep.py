@@ -8,7 +8,7 @@ vanish.  Windows 5..25, 1..10 views, n_best 1..3, both combinations, 8-bit and f
 must agree bit for bit (NaN counts as equal to NaN; the ratio is not compared for V = 1, where the reference reads an
 uninitialised slot, SURVEY Q8).
 
-    python tools/gpu_cost_sweep.py [configs] [pairs]   ->  gpurun_out/r02_cost_sweep.json
+    python tools/gpu_cost_sweep.py [configs] [pairs]   ->  $TSAR_RECORD_DIR/cost_sweep.json
 """
 import json
 import os
@@ -78,6 +78,6 @@ for trial in range(NCFG):
     bad += 0 if ok else 1
     rows.append(row)
     print(("ok  " if ok else "FAIL"), json.dumps(row), flush=True)
-json.dump(dict(configs=NCFG, exact_configs=NCFG - bad, rows=rows), open(os.path.join(ROOT, "gpurun_out", "r02_cost_sweep.json"), "w"), indent=1)
+pc.record("cost_sweep.json", dict(configs=NCFG, exact_configs=NCFG - bad, rows=rows))
 print(f"{NCFG - bad} of {NCFG} configurations exact")
 sys.exit(1 if bad else 0)

@@ -5,7 +5,7 @@ ADVERSARIAL state: random planes (incl. degenerate normals and plane offsets of 
 around the thresholds (0, 2.0 = MAXCOST), random best views, random reliable flags, random region labels and region tables
 whose planes include zeros, on random sizes and camera rigs.  Every field is compared bit for bit (NaN payloads included).
 
-    python tools/gpu_glue_sweep.py [N]   ->  gpurun_out/r02_glue_sweep.json
+    python tools/gpu_glue_sweep.py [N]   ->  $TSAR_RECORD_DIR/glue_sweep.json
 """
 import json
 import os
@@ -81,6 +81,6 @@ for trial in range(N):
     bad += 0 if ok else 1
     rows.append(row)
     print(("ok  " if ok else "FAIL"), json.dumps(row), flush=True)
-json.dump(dict(trials=N, bit_exact_trials=N - bad, rows=rows), open(os.path.join(ROOT, "gpurun_out", "r02_glue_sweep.json"), "w"), indent=1)
+pc.record("glue_sweep.json", dict(trials=N, bit_exact_trials=N - bad, rows=rows))
 print(f"{N - bad} of {N} trials bit-exact")
 sys.exit(1 if bad else 0)

@@ -6,7 +6,7 @@ exactly collinear points, outlier fractions 0 ... 60 %, several weak regions per
 host-supplied and the device-generated stream.  Planes must agree bit for bit (a NaN on both sides counts as equal).
 Regions without any reliable point are left out: the reference divides by zero there (rand() % 0).
 
-    python tools/gpu_ransac_sweep.py [N]   ->  gpurun_out/r02_ransac_sweep.json
+    python tools/gpu_ransac_sweep.py [N]   ->  $TSAR_RECORD_DIR/ransac_sweep.json
 """
 import json
 import os
@@ -17,10 +17,10 @@ import numpy as np
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 from tests import parity_common as pc  # noqa: E402
-from oracle import ref_host_binding as rh  # noqa: E402
 
 N = int(sys.argv[1]) if len(sys.argv) > 1 else 30
 pkg = pc.load_pkg()
+rh = pc.ref_host()
 L = pkg._lib
 rng = np.random.RandomState(int(os.environ.get("TSAR_SWEEP_SEED", "2718")))   # TSAR_SWEEP_SEED: another campaign
 rows, bad = [], 0
@@ -80,6 +80,6 @@ for trial in range(N):
     rows.append(row)
     print(("ok  " if ok else "FAIL"), json.dumps({k: v for k, v in row.items() if k not in ("mine", "ref")}), flush=True)
 mine.close()
-json.dump(dict(trials=N, exact_trials=N - bad, rows=rows), open(os.path.join(ROOT, "gpurun_out", "r02_ransac_sweep.json"), "w"), indent=1)
+pc.record("ransac_sweep.json", dict(trials=N, exact_trials=N - bad, rows=rows))
 print(f"{N - bad} of {N} trials exact")
 sys.exit(1 if bad else 0)

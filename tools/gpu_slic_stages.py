@@ -4,10 +4,9 @@
   * superpixel records (centre, colour, pixel count) after 0..5 iterations on a piecewise-constant image (exact ties
     in the distance, where a last-ulp difference decides) and on a noise image, bit for bit.
 
-    python tools/gpu_slic_stages.py   ->  gpurun_out/r02_slic_stages.json
+    python tools/gpu_slic_stages.py   ->  $TSAR_RECORD_DIR/slic_stages.json
 """
 import ctypes as C
-import json
 import os
 import sys
 
@@ -19,9 +18,6 @@ from tests import parity_common as pc  # noqa: E402
 
 pkg = pc.load_pkg()
 rb = pc.ref_binding()
-rl = C.CDLL(os.path.join(ROOT, "oracle", "_ref", "libgslic_ref.so"))
-rl.ref_slic_last_lab.restype = C.c_longlong
-rl.ref_slic_last_lab.argtypes = [C.c_void_p, C.c_longlong]
 eng = pkg.DepthmapEngine(0)
 eng.lib.tsar_dbg_slic_lab.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t]
 res = {}
@@ -32,11 +28,10 @@ v = np.arange(n * n, dtype=np.uint32)
 img = np.zeros((n, n, 4), np.uint8)
 img[..., 0] = (v & 255).reshape(n, n); img[..., 1] = ((v >> 8) & 255).reshape(n, n); img[..., 2] = ((v >> 16) & 255).reshape(n, n)
 mine_lab = np.empty((n, n, 4), np.float32)
-ref_lab = np.empty((n, n, 4), np.float32)
 lm = eng.slic(img, spixel_size=20, no_iters=0)
 eng._ck(eng.lib.tsar_dbg_slic_lab(eng.h, mine_lab.ctypes.data, n * n), "lab")
 lr, _ = rb.ref_slic(img, spixel_size=20, no_iters=0)
-rl.ref_slic_last_lab(ref_lab.ctypes.data, n * n)
+ref_lab = rb.slic_last_lab(n * n).reshape(n, n, 4)
 eq = (mine_lab[..., :3].view(np.uint32) == ref_lab[..., :3].view(np.uint32)).all(-1)
 res["rgb2CIELab_all_16777216_colours_bit_exact"] = float(eq.mean())
 res["labels_on_that_image_identical"] = float((lm == lr).mean())
@@ -58,15 +53,14 @@ for name in ("blocks", "noise"):
         mc = np.zeros((nsp, 8), np.float32); cnt = C.c_int(0)
         eng._ck(eng.lib.tsar_dbg_slic_centres(eng.h, mc.ctypes.data_as(C.c_void_p), nsp, C.byref(cnt)), "centres")
         r, _ = rb.ref_slic(bgrx, spixel_size=size, no_iters=it, coh_weight=10.0)
-        rc = np.zeros((nsp, 8), np.float32)
-        rl.ref_slic_last_centres(rc.ctypes.data_as(C.c_void_p), nsp)
+        rc = rb.slic_last_centres(nsp)
         sel = [0, 1, 2, 3, 4, 6, 7]          # colour w is not defined by the reference's conversion
         rows.append(dict(iterations=it, labels_identical=float((m == r).mean()),
                          records_bit_exact=float((mc.view(np.uint32)[:, sel] == rc.view(np.uint32)[:, sel]).all(1).mean())))
         print(name, rows[-1], flush=True)
     res[name] = rows
 eng.close()
-json.dump(res, open(os.path.join(ROOT, "gpurun_out", "r02_slic_stages.json"), "w"), indent=1)
+pc.record("slic_stages.json", res)
 ok = res["rgb2CIELab_all_16777216_colours_bit_exact"] == 1.0 and all(r["labels_identical"] == 1.0 and r["records_bit_exact"] == 1.0 for k in ("blocks", "noise") for r in res[k])
 print("ALL EXACT" if ok else "MISMATCH")
 sys.exit(0 if ok else 1)

@@ -3,7 +3,7 @@
 random image sizes (incl. sizes that are not multiples of the superpixel size), superpixel sizes, iteration counts,
 coherence weights, with and without the connectivity pass, on structured and on noise images.  Labels must be identical.
 
-    python tools/gpu_slic_sweep.py [N]   ->  gpurun_out/r02_slic_sweep.json
+    python tools/gpu_slic_sweep.py [N]   ->  $TSAR_RECORD_DIR/slic_sweep.json
 """
 import json
 import os
@@ -48,6 +48,6 @@ for trial in range(N):
     rows.append(row)
     print(("ok  " if same == 1.0 else "FAIL"), json.dumps(row), flush=True)
 eng.close()
-json.dump(dict(trials=N, identical_trials=N - bad, rows=rows), open(os.path.join(ROOT, "gpurun_out", "r02_slic_sweep.json"), "w"), indent=1)
+pc.record("slic_sweep.json", dict(trials=N, identical_trials=N - bad, rows=rows))
 print(f"{N - bad} of {N} configurations identical")
 sys.exit(1 if bad else 0)

@@ -5,7 +5,7 @@ variable uninitialised when a median is never reached): random sizes, reliable-p
 masks give the tiny neighbour lists where medians are not reached), random region tables, planes straight from a short
 PatchMatch run.  Every level starts from the reference's state; flags, planes and disparities must agree on 100 % of the pixels.
 
-    python tools/gpu_wmf_sweep.py [N]   ->  gpurun_out/r02_wmf_sweep.json
+    python tools/gpu_wmf_sweep.py [N]   ->  $TSAR_RECORD_DIR/wmf_sweep.json
 """
 import json
 import os
@@ -62,6 +62,6 @@ for trial in range(N):
     bad += 0 if ok else 1
     rows.append(row)
     print(("ok  " if ok else "FAIL"), json.dumps(row), flush=True)
-json.dump(dict(trials=N, exact_trials=N - bad, rows=rows), open(os.path.join(ROOT, "gpurun_out", "r02_wmf_sweep.json"), "w"), indent=1)
+pc.record("wmf_sweep.json", dict(trials=N, exact_trials=N - bad, rows=rows))
 print(f"{N - bad} of {N} trials exact")
 sys.exit(1 if bad else 0)
