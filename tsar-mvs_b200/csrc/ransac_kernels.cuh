@@ -16,7 +16,7 @@
 // draws them from rand()/system_clock (not reproducible); the caller supplies the stream instead (the values
 // rand() would have returned, 46 000 per region) or a seed for a device-generated stream (ransac_rand_kernel).
 // Kept quirks: the A coefficient of calcLinePara uses (y3-y1) twice (main.cpp:159); ties (>=) replace the best.
-// Deviation: when a region has more than 49 999 reliable pixels the reference keeps a random subset
+// Deviation: when a region has more than 50 000 reliable pixels the reference keeps a random subset of 49 999
 // (std::shuffle with a clock seed); we keep an evenly strided subset.
 #pragma once
 #include <cooperative_groups.h>
