@@ -201,7 +201,7 @@ int tsar_download(tsar_ctx *ctx, int field, void *host_dst, size_t bytes);
  * written by the reference).  The output layout is split on the device; host pointers (pinned memory makes the copies
  * asynchronous to other streams); any of them may be NULL. */
 int tsar_download_outputs(tsar_ctx *ctx, float *depth_out, float *normals_out, float *confid_out);
-/* Device pointer of a field (for zero-copy consumers such as a fusion stage on the same GPU).  For TSAR_F_NORM4 and
+/* Device pointer of a field (for zero-copy consumers on the same GPU).  For TSAR_F_NORM4 and
  * TSAR_F_COST the per-colour double buffers are first merged into the returned array (on the context's stream); the
  * pointer is valid until the next call that launches propagation or refinement (tsar_launch, tsar_iterate,
  * tsar_depthmap), after which the live values of one colour sit in the other buffer again. */
@@ -265,6 +265,43 @@ int tsar_dbg_candidate_stats(tsar_ctx *ctx, int colour, unsigned long long *out2
  * by nvcc with the loop-hoisted form (fma(m1,y, m0*x) + m2); wrapper_rounding=1 selects that form so the
  * unit-level test can require bit equality against the wrapper.  Production kernels are unaffected. */
 int tsar_dbg_eval_rounding(tsar_ctx *ctx, int wrapper_rounding);
+
+/* ---- multi-view fusion (DESIGN.md section 4.6) ------------------------------------------------------------------------
+ * Fuses the per-view depth maps of a dataset (TSAR_disp.dmb / TSAR_normals.dmb + the colour images) into one coloured
+ * point cloud by a multi-view consistency check.  The stage of the reference pipeline after TSAR is Fusion.exe, a closed
+ * binary; this rule follows the published ACMM/ACMMP RunFusion family with the differences listed in DESIGN.md 4.6.
+ * A handle of its own, since fusion spans many views and a tsar_ctx holds one.  All views have the same W x H.
+ * Views are fused in index order (view v skips source pixels that views < v already used); inside a view the work is
+ * parallel and the result identical to the sequential rule.  Device memory: 21 B per pixel and view (depth + normal
+ * float4, BGR + pad, mask) plus scratch for one view (8 B per pixel and neighbour, 29 B per pixel); the points leave the
+ * device view by view. */
+#define TSAR_FUSION_MAX_NEIGHBOURS 32
+
+typedef struct tsar_view_camera { float K[9], R[9], t[3]; } tsar_view_camera;   /* world -> camera, row-major */
+typedef struct tsar_fusion_params {
+    float max_reproj_px;   /* 2.0   round-trip reprojection error, pixels (strict <)                  */
+    float max_rel_depth;   /* 0.01  |z' - D| < max_rel_depth * D (strict)                              */
+    float max_normal_deg;  /* 10    n_v.n_u >= cos(max_normal_deg) |n_v| |n_u| (cosine taken in double) */
+    int min_consistent;    /* 2     consistent source pixels a point needs                             */
+} tsar_fusion_params;
+typedef struct tsar_fusion tsar_fusion;
+
+/* `stream` as in tsar_create.  TSAR_ERR_ARG unless n_views >= 1 and 1 <= W*H <= 0x7f7f7f7f - 256; TSAR_ERR_NODEVICE
+ * without an sm_100 device, TSAR_ERR_NOMEM when the views do not fit. */
+int tsar_fusion_create(int device, void *stream, int n_views, int W, int H, tsar_fusion **out);
+/* Host pointers: depth = W*H floats (camera z, 0 = no depth; a pixel is used when its depth is finite and > 0),
+ * normals = W*H*3 floats (world frame), bgr = W*H*3 bytes.  neighbours = 1..32 distinct view indices, not `view`. */
+int tsar_fusion_set_view(tsar_fusion *f, int view, const tsar_view_camera *cam, const float *depth,
+                         const float *normals, const unsigned char *bgr, const int *neighbours, int n_neighbours);
+/* Fuses every view (all must be set; masks are reset first, so it may be called again with other parameters).
+ * n_points (may be NULL) receives the number of points, ordered by view, then by raster order of the reference pixel. */
+int tsar_fusion_run(tsar_fusion *f, const tsar_fusion_params *p, long long *n_points);
+/* The points of the last run: xyz and normals 3 floats, rgb 3 bytes each; TSAR_ERR_ARG when capacity < n_points. */
+int tsar_fusion_points(tsar_fusion *f, float *xyz, float *normals, unsigned char *rgb, long long capacity);
+int tsar_fusion_destroy(tsar_fusion *f);
+const char *tsar_fusion_last_error(const tsar_fusion *f);
+/* Resolution rounds of the last run: the most any view needed and the sum over the views (data-dependent). */
+int tsar_fusion_dbg_rounds(const tsar_fusion *f, int *max_rounds, long long *total_rounds);
 
 #ifdef __cplusplus
 }

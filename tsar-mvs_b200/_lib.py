@@ -40,6 +40,17 @@ class TsarSlicSettings(C.Structure):
     ]
 
 
+class TsarViewCamera(C.Structure):
+    """tsar_view_camera: world -> camera K, R, t of one view (row-major)."""
+    _fields_ = [("K", C.c_float * 9), ("R", C.c_float * 9), ("t", C.c_float * 3)]
+
+
+class TsarFusionParams(C.Structure):
+    """tsar_fusion_params (DESIGN.md section 4.6)."""
+    _fields_ = [("max_reproj_px", C.c_float), ("max_rel_depth", C.c_float), ("max_normal_deg", C.c_float),
+                ("min_consistent", C.c_int)]
+
+
 # tsar_field
 F_NORM4, F_COST, F_DEPTH, F_FAKEDEPTH, F_SCALE, F_CANNY, F_RATIO, F_BEVIEW, F_LRDIFF, F_CONFID, \
     F_REGION_TEXT, F_REGION_NORM4 = range(12)
@@ -53,6 +64,8 @@ EXPORTS = [
     "tsar_wmf_final", "tsar_set_regions", "tsar_fit_region_planes", "tsar_fit_region_planes_seeded", "tsar_ransac_rand_value", "tsar_ransac_rand_per_region", "tsar_upload", "tsar_download", "tsar_device_ptr", "tsar_depthmap",
     "tsar_depthmap_host", "tsar_slic", "tsar_launch_count", "tsar_eval_count", "tsar_version", "tsar_dbg_tex_sample", "tsar_dbg_peaks", "tsar_dbg_eval_rounding", "tsar_dbg_candidate_stats", "tsar_dbg_tex_formats", "tsar_profile", "tsar_profile_read",
     "tsar_weak_edges", "tsar_weak_connect", "tsar_weak_boundary", "tsar_weak_close_border", "tsar_weak_regions", "tsar_set_labels_quarter", "tsar_scale_from_weak_png", "tsar_scale_from_confidence", "tsar_download_outputs",
+    "tsar_fusion_create", "tsar_fusion_set_view", "tsar_fusion_run", "tsar_fusion_points", "tsar_fusion_destroy",
+    "tsar_fusion_last_error", "tsar_fusion_dbg_rounds",
 ]
 
 
@@ -121,6 +134,13 @@ def load():
         "tsar_scale_from_weak_png": (i, [vp, vp]),
         "tsar_scale_from_confidence": (i, [vp, C.c_float]),
         "tsar_download_outputs": (i, [vp, vp, vp, vp]),
+        "tsar_fusion_create": (i, [i, vp, i, i, i, C.POINTER(vp)]),
+        "tsar_fusion_set_view": (i, [vp, i, C.POINTER(TsarViewCamera), vp, vp, vp, ip, i]),
+        "tsar_fusion_run": (i, [vp, C.POINTER(TsarFusionParams), C.POINTER(C.c_longlong)]),
+        "tsar_fusion_points": (i, [vp, vp, vp, vp, C.c_longlong]),
+        "tsar_fusion_destroy": (i, [vp]),
+        "tsar_fusion_last_error": (C.c_char_p, [vp]),
+        "tsar_fusion_dbg_rounds": (i, [vp, ip, C.POINTER(C.c_longlong)]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(lib, name)

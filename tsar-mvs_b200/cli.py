@@ -21,6 +21,9 @@ HoughLinesP / line as the reference uses OpenCV) labels the reference view; regi
 tsar_fit_region_planes and are completed by update_scale(_2).  `-no_weak_texture` skips it; `-regions_file labels.npy`
 (+ `-regions_text text.npy`) supplies a precomputed label map instead.
 `-write_ply` also writes `TSAR_model.ply` (displayUtils.h:77-158).
+`-fuse` fuses every view's `APD/<stem>/TSAR_disp.dmb` + `TSAR_normals.dmb` with the colour images, cams and pair.txt
+into one point cloud, `<mslp>/TSAR_fused.ply` (fusion.py, DESIGN.md section 4.6; one GPU, views in dataset order).
+With `-all_views` it runs after the last view (single process only: fusion reads every view's output).
 Extra: `--synthetic=<C1|C2|small|tiny>` first writes a synthetic dataset in the reference's folder layout.
 
 `-all_views` replaces the per-view process loop of the run scripts (scripts/pipes.sh:30-49): every image of the
@@ -31,6 +34,7 @@ contiguous blocks over the ranks (shard.py), one GPU per rank, no collective.  `
 output files are already complete (an interrupted run continues where it stopped; files are written under a temporary
 name and renamed, so a partial file never counts).
 """
+import itertools
 import os
 import sys
 
@@ -44,14 +48,14 @@ NUMERIC = {"blocksize", "iterations", "n_best", "cost_gamma", "depth_min", "dept
            "self_similarity_n", "good_factor", "num_img_processed", "seed", "synthetic", "device", "lanes", "io_threads"}
 PATHS = {"images_folder", "mslp_folder", "krt_file", "output_folder", "p_folder", "camera_folder", "calib_file", "pmvs_folder",
          "bounding_folder", "regions_file", "regions_text", "regions_size"}
-BOOLS = {"color_processing", "view_selection", "import_apd", "no_display", "all_views", "no_weak_texture", "write_ply", "wmf", "no_slic", "no_write", "resume"}
+BOOLS = {"color_processing", "view_selection", "import_apd", "no_display", "all_views", "no_weak_texture", "write_ply", "wmf", "no_slic", "no_write", "resume", "fuse"}
 
 
 def parse_args(argv):
     """getParametersFromCommandLine (main.cpp:708-1009), tolerant in the same places."""
     opt = dict(images=[], blocksize=19, iterations=8, n_best=2, cost_comb=1, cam_scale=1.0, depth_min=-1.0, depth_max=-1.0,
                seed=20240601, device=0, images_folder="", mslp_folder="", output_folder="", synthetic=None,
-               color_processing=False, import_apd=False, all_views=False, no_weak_texture=False, write_ply=False, wmf=False, no_slic=False, no_write=False, resume=False,
+               color_processing=False, import_apd=False, all_views=False, no_weak_texture=False, write_ply=False, wmf=False, no_slic=False, no_write=False, resume=False, fuse=False,
                regions_file=None, regions_text=None, regions_size=None, lanes=2, io_threads=4)
     i = 0
     while i < len(argv):
@@ -275,8 +279,16 @@ def run(argv):
         opt["images"] = opt["images"] or names
         opt["images_folder"] = os.path.join(mslp, "images/")
     if opt["all_views"]:
+        if opt["fuse"] and int(os.environ.get("WORLD_SIZE", "1")) > 1:
+            print("[tsar_cli] -fuse runs on one GPU (view v depends on the views before it): run -all_views under several "
+                  "ranks without -fuse, then `tsar_cli.py -fuse -mslp_folder ...` as a single process", file=sys.stderr)
+            return 2
         run_all_views(opt, mslp)
+        if opt["fuse"]:
+            return run_fuse(opt, mslp)
         return 0
+    if opt["fuse"]:
+        return run_fuse(opt, mslp)
     if not opt["images"]:
         print(__doc__)
         return 2
@@ -344,6 +356,77 @@ def read_pair_table(path):
         tok = lines[2 * k + 2].split()
         table[cam] = [int(tok[1 + 2 * j]) for j in range(int(tok[0]))]
     return table
+
+
+def read_fusion_views(opt, mslp, lazy=False):
+    """The inputs of fusion.fuse for every image of the dataset (names as -all_views lists them): depth and normals from
+    APD/<stem>/, K R t from cams/ (cam_scale applied), the colour image, and the pair.txt neighbours that exist in the
+    dataset.  Raises FileNotFoundError naming every view whose outputs are missing, ValueError when there is no image or
+    naming every view with no neighbour in the dataset or more than 32.  lazy=True returns (number of views, generator
+    of the views) so that only one view is held in host memory at a time."""
+    import cv2
+    from .fusion import MAX_NEIGHBOURS
+    folder = opt["images_folder"] or os.path.join(mslp, "images/")
+    names = opt["images"] or sorted(n for n in os.listdir(folder) if n.lower().endswith((".jpg", ".jpeg", ".png", ".npy")))
+    if not names:
+        raise ValueError(f"no images in {folder}")
+    apd = [os.path.join(mslp, "APD", n[:8]) for n in names]
+    missing = [n[:8] for n, d in zip(names, apd) if not all(os.path.exists(os.path.join(d, f)) for f in ("TSAR_disp.dmb", "TSAR_normals.dmb"))]
+    if missing:
+        raise FileNotFoundError(f"no TSAR_disp.dmb / TSAR_normals.dmb under {os.path.join(mslp, 'APD')} for view(s) {', '.join(missing)}: "
+                                f"compute them first (-all_views)")
+    ids = [int(n[4:8]) for n in names]
+    by_id = {c: k for k, c in enumerate(ids)}
+    pairs = read_pair_table(os.path.join(mslp, "pair.txt"))
+    neighbours = [[by_id[c] for c in pairs.get(i, []) if c in by_id] for i in ids]
+    bad = [f"{n[:8]} ({len(nb)})" for n, nb in zip(names, neighbours) if not 1 <= len(nb) <= MAX_NEIGHBOURS]
+    if bad:
+        raise ValueError(f"fusion needs 1..{MAX_NEIGHBOURS} pair.txt neighbours present in the dataset per view; "
+                         f"view(s) {', '.join(bad)} have not")
+
+    def load(k):
+        n = names[k]
+        K, R, t, _, _ = read_cam_txt(os.path.join(mslp, "cams", f"{n[:8]}_cam.txt"))
+        K = K.copy()
+        K[:2] /= opt["cam_scale"]
+        path = os.path.join(folder, n)
+        if n.endswith(".npy"):
+            bgr = np.repeat(np.clip(np.load(path), 0, 255).astype(np.uint8)[..., None], 3, axis=-1)
+        else:
+            bgr = cv2.imread(path, cv2.IMREAD_COLOR)
+            if bgr is None:
+                raise FileNotFoundError(path)
+        return dict(K=K, R=R, t=t, depth=dmb.read_dmb(os.path.join(apd[k], "TSAR_disp.dmb")),
+                    normals=dmb.read_dmb(os.path.join(apd[k], "TSAR_normals.dmb")), bgr=bgr,
+                    neighbours=neighbours[k])
+
+    if lazy:
+        return len(names), (load(k) for k in range(len(names)))
+    return [load(k) for k in range(len(names))]
+
+
+def run_fuse(opt, mslp, quiet=False):
+    """-fuse: every view's depth + normal maps -> <mslp>/TSAR_fused.ply.  Returns the exit code."""
+    import time
+    from . import fusion
+    t0 = time.perf_counter()
+    from .engine import TsarError
+    try:
+        n_views, views = read_fusion_views(opt, mslp, lazy=True)
+        first = next(views)
+        H, W = first["depth"].shape
+        with fusion.FusionEngine(n_views, W, H, device=int(opt["device"])) as eng:
+            for k, v in enumerate(itertools.chain([first], views)):
+                eng.set_view(k, v["K"], v["R"], v["t"], v["depth"], v["normals"], v["bgr"], v["neighbours"])
+            xyz, nrm, rgb = eng.run()
+    except (FileNotFoundError, ValueError, TsarError) as e:    # set_view names the view (index in dataset order)
+        print(f"[tsar_cli] -fuse: {e}", file=sys.stderr)
+        return 1
+    out = os.path.join(mslp, "TSAR_fused.ply")
+    dmb.write_fused_ply(out, xyz, nrm, rgb)
+    if not quiet:
+        print(f"[tsar_cli] fused {n_views} views ({W}x{H}) into {len(xyz)} points in {time.perf_counter() - t0:.2f} s -> {out}")
+    return 0
 
 
 _LANE_POOL = {}   # (device, W, H) -> lanes kept alive between run_all_views calls of one process (persistent=True)

@@ -3,6 +3,8 @@ int32 height, int32 width, int32 channels, then h*w*channels float32 row-major. 
 scripts consume TSAR_disp.dmb (1 channel) and TSAR_normals.dmb (3 channels) (main.cpp:1807-1861)."""
 import numpy as np
 
+PLY_VERTEX = [("p", "<f4", 3), ("n", "<f4", 3), ("c", "u1", 3)]   # float x y z, float nx ny nz, uchar red green blue
+
 
 def write_dmb(path, arr):
     a = np.ascontiguousarray(arr, np.float32)
@@ -51,19 +53,30 @@ def write_model_ply(path, depth, normals, gray, K, R, t):
         X = (rhs @ Minv.T).astype(np.float32)
     bad = ~np.isfinite(X).all(-1)
     X[bad] = 0.0
-    rec = np.zeros(W * H, dtype=[("p", "<f4", 3), ("n", "<f4", 3), ("c", "u1", 3)])
+    rec = np.zeros(W * H, dtype=PLY_VERTEX)
     rec["p"] = X.reshape(-1, 3)
     rec["n"] = np.asarray(normals, np.float32).transpose(1, 0, 2).reshape(-1, 3)
     rec["c"] = np.asarray(gray).astype(np.uint8).T.reshape(-1, 1)
+    _write_vertices(path, rec)
+
+
+def write_fused_ply(path, xyz, normals, rgb):
+    """The fused point cloud (fusion.fuse) in the vertex layout of TSAR_model.ply; read_model_ply reads it back."""
+    rec = np.zeros(len(np.asarray(xyz).reshape(-1, 3)), dtype=PLY_VERTEX)
+    rec["p"], rec["n"], rec["c"] = (np.asarray(a, dt).reshape(-1, 3) for a, dt in ((xyz, np.float32), (normals, np.float32), (rgb, np.uint8)))
+    _write_vertices(path, rec)
+
+
+def _write_vertices(path, rec):
     with open(path, "wb") as f:
-        f.write(("ply\nformat binary_little_endian 1.0\n" + f"element vertex {H * W}\n" +
+        f.write(("ply\nformat binary_little_endian 1.0\n" + f"element vertex {len(rec)}\n" +
                  "property float x\nproperty float y\nproperty float z\nproperty float nx\nproperty float ny\nproperty float nz\n"
                  "property uchar red\nproperty uchar green\nproperty uchar blue\nend_header\n").encode())
         rec.tofile(f)
 
 
 def read_model_ply(path):
-    """Reader for the file above (tests / hand-over to a fusion stage): returns (points [n][3], normals, grey)."""
+    """Reader for TSAR_model.ply and TSAR_fused.ply: returns (points [n][3], normals, colour)."""
     with open(path, "rb") as f:
         n = None
         while True:
@@ -72,5 +85,5 @@ def read_model_ply(path):
                 n = int(line.split()[-1])
             if line == "end_header":
                 break
-        rec = np.fromfile(f, dtype=[("p", "<f4", 3), ("n", "<f4", 3), ("c", "u1", 3)], count=n)
+        rec = np.fromfile(f, dtype=PLY_VERTEX, count=n)
     return rec["p"], rec["n"], rec["c"]
