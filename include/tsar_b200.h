@@ -238,6 +238,9 @@ int tsar_eval_count(tsar_ctx *ctx, int iters, long long *n_evals);
  * stream it is launched on: enable, run, then read the summed duration and the number of launches. */
 int tsar_profile(tsar_ctx *ctx, int enable);
 int tsar_profile_read(tsar_ctx *ctx, float *checker_ms_total, int *n_launches);
+/* The same events one by one: ms[i] = CUDA-event time of the i-th checkerboard launch since profiling was enabled (the
+ * first cap of them); *n_launches = how many there were.  Consumes the events as tsar_profile_read does. */
+int tsar_profile_read_launches(tsar_ctx *ctx, float *ms, int cap, int *n_launches);
 const char *tsar_version(void);
 /* tex2D<float> of image `image` at n unnormalised coordinates (xy = n float2, host): used to
  * calibrate software models of the texture unit's bilinear filter (SURVEY Q9). */
@@ -265,6 +268,12 @@ int tsar_dbg_candidate_stats(tsar_ctx *ctx, int colour, unsigned long long *out2
  * by nvcc with the loop-hoisted form (fma(m1,y, m0*x) + m2); wrapper_rounding=1 selects that form so the
  * unit-level test can require bit equality against the wrapper.  Production kernels are unaffected. */
 int tsar_dbg_eval_rounding(tsar_ctx *ctx, int wrapper_rounding);
+
+/* Quad-cooperative sampling (DESIGN.md 4.2): the four lanes of a texture quad fetch samples of one window at a time.
+ * checker_launches < 0: off everywhere (as env TSAR_B200_NO_QUAD_SAMPLING=1); >= 0: used by tsar_init_planes and by
+ * the first checker_launches checkerboard launches after tsar_init_planes / tsar_load_planes.  Applies to the 11x11
+ * window with 8-bit textures (and, for the checkerboard, pinhole cameras).  Results are bit-identical either way. */
+int tsar_dbg_quad_sampling(tsar_ctx *ctx, int checker_launches);
 
 /* ---- multi-view fusion (DESIGN.md section 4.6) ------------------------------------------------------------------------
  * Fuses the per-view depth maps of a dataset (TSAR_disp.dmb / TSAR_normals.dmb + the colour images) into one coloured

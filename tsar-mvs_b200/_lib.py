@@ -62,7 +62,7 @@ EXPORTS = [
     "tsar_init_planes", "tsar_load_planes", "tsar_launch", "tsar_iterate", "tsar_eval_planes", "tsar_lrdiff",
     "tsar_getview", "tsar_get_disp", "tsar_update_scale_2", "tsar_update_scale", "tsar_compute_disp", "tsar_wmf",
     "tsar_wmf_final", "tsar_set_regions", "tsar_fit_region_planes", "tsar_fit_region_planes_seeded", "tsar_ransac_rand_value", "tsar_ransac_rand_per_region", "tsar_upload", "tsar_download", "tsar_device_ptr", "tsar_depthmap",
-    "tsar_depthmap_host", "tsar_slic", "tsar_launch_count", "tsar_eval_count", "tsar_version", "tsar_dbg_tex_sample", "tsar_dbg_peaks", "tsar_dbg_eval_rounding", "tsar_dbg_candidate_stats", "tsar_dbg_tex_formats", "tsar_profile", "tsar_profile_read",
+    "tsar_depthmap_host", "tsar_slic", "tsar_launch_count", "tsar_eval_count", "tsar_version", "tsar_dbg_tex_sample", "tsar_dbg_peaks", "tsar_dbg_eval_rounding", "tsar_dbg_quad_sampling", "tsar_dbg_candidate_stats", "tsar_dbg_tex_formats", "tsar_profile", "tsar_profile_read", "tsar_profile_read_launches",
     "tsar_weak_edges", "tsar_weak_connect", "tsar_weak_boundary", "tsar_weak_close_border", "tsar_weak_regions", "tsar_set_labels_quarter", "tsar_scale_from_weak_png", "tsar_scale_from_confidence", "tsar_download_outputs",
     "tsar_fusion_create", "tsar_fusion_set_view", "tsar_fusion_run", "tsar_fusion_points", "tsar_fusion_destroy",
     "tsar_fusion_last_error", "tsar_fusion_dbg_rounds",
@@ -121,10 +121,12 @@ def load():
         "tsar_dbg_tex_sample": (i, [vp, i, i, vp, vp]),
         "tsar_dbg_peaks": (i, [vp, fp]),
         "tsar_dbg_eval_rounding": (i, [vp, i]),
+        "tsar_dbg_quad_sampling": (i, [vp, i]),
         "tsar_dbg_candidate_stats": (i, [vp, i, vp]),
         "tsar_dbg_tex_formats": (i, [vp, i, i, vp, vp, vp]),
         "tsar_profile": (i, [vp, i]),
         "tsar_profile_read": (i, [vp, fp, ip]),
+        "tsar_profile_read_launches": (i, [vp, fp, i, ip]),
         "tsar_weak_edges": (i, [vp, i, i, i, vp]),
         "tsar_weak_connect": (i, [vp, i, i, vp, vp, i, ip]),
         "tsar_weak_boundary": (i, [vp, i, i, i, vp]),

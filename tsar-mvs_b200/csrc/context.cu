@@ -35,6 +35,10 @@ struct RansacScratch {
     int nt_cap = 0, grid = 0;
 };
 
+// Checkerboard launches after the planes were set that use quad-cooperative sampling (the rest use the per-lane
+// loop).  Chosen by measurement, DESIGN.md 4.4.
+constexpr int kQuadLaunches = 2;
+
 struct tsar_ctx {
     int device = 0;
     cudaStream_t stream = nullptr;
@@ -90,6 +94,10 @@ struct tsar_ctx {
     long long launches = 0;
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;
     bool fused = true;
+    // quad-cooperative sampling (pm_core.cuh, view_cost_quad) for the initialisation and the first quad_launches
+    // checkerboard launches after the planes were set; -1 (env TSAR_B200_NO_QUAD_SAMPLING=1): never
+    int quad_launches = kQuadLaunches;
+    int checker_since_planes = 0;
     int eval_wrapper_rounding = 0;  // test-only, see tsar_dbg_eval_rounding
     bool profiling = false;
     std::vector<std::pair<cudaEvent_t, cudaEvent_t>> prof_events;  // around every checkerboard kernel
@@ -325,7 +333,9 @@ static int launch_checker(tsar_ctx *ctx, int mode, int colour, const uint32_t *r
         CK(cudaEventCreate(&p0)); CK(cudaEventCreate(&p1));
         CK(cudaEventRecord(p0, ctx->stream));
     }
-    CK(ctx->variant->checker(ctx->use_u8, mode, ctx->pm, ctx->ref_img, a, ctx->stream));
+    const int quad = ctx->checker_since_planes < ctx->quad_launches && ctx->variant->has_quad && ctx->use_u8 && ctx->pm.k_pinhole;
+    CK(ctx->variant->checker(ctx->use_u8, quad, mode, ctx->pm, ctx->ref_img, a, ctx->stream));
+    ctx->checker_since_planes++;
     if (ctx->profiling) {
         CK(cudaEventRecord(p1, ctx->stream));
         ctx->prof_events.emplace_back(p0, p1);
@@ -380,6 +390,8 @@ int tsar_create(int device, void *stream, tsar_ctx **out) {
     ctx->fused = !(uf && uf[0] == '1');
     const char *n8 = getenv("TSAR_B200_NO_U8");
     ctx->allow_u8 = !(n8 && n8[0] == '1');
+    const char *nq = getenv("TSAR_B200_NO_QUAD_SAMPLING");
+    if (nq && nq[0] == '1') ctx->quad_launches = -1;
     *out = ctx;
     return TSAR_OK;
 }
@@ -569,8 +581,10 @@ int tsar_init_planes(tsar_ctx *ctx, uint64_t seed) {
     if (rc) return rc;
     if ((rc = zero_state(ctx, false))) return rc;
     if ((rc = make_rng_table(ctx, seed))) return rc;
-    CK(ctx->variant_init->init(ctx->use_u8, ctx->pm_init, ctx->ref_img, ctx->rng, ctx->rng_len, ctx->plane[0], ctx->cost[0], ctx->stream));
+    const int quad = ctx->quad_launches >= 0 && ctx->variant_init->has_quad && ctx->use_u8;
+    CK(ctx->variant_init->init(ctx->use_u8, quad, ctx->pm_init, ctx->ref_img, ctx->rng, ctx->rng_len, ctx->plane[0], ctx->cost[0], ctx->stream));
     ctx->launches++;
+    ctx->checker_since_planes = 0;
     ctx->cur[0] = ctx->cur[1] = 0;
     ctx->have_planes = true;
     return seed_alt_buffers(ctx);
@@ -588,6 +602,7 @@ int tsar_load_planes(tsar_ctx *ctx, const float *norm4, const float *cost) {
         ctx->launches++;
     }
     CK(cudaStreamSynchronize(ctx->stream));
+    ctx->checker_since_planes = 0;
     ctx->cur[0] = ctx->cur[1] = 0;
     ctx->have_planes = true;
     return seed_alt_buffers(ctx);
@@ -1182,6 +1197,22 @@ int tsar_profile_read(tsar_ctx *ctx, float *checker_ms_total, int *n_launches) {
     return TSAR_OK;
 }
 
+int tsar_profile_read_launches(tsar_ctx *ctx, float *ms, int cap, int *n_launches) {
+    if (!ctx || !n_launches || cap < 0 || (cap > 0 && !ms)) return TSAR_ERR_ARG;
+    CK(cudaStreamSynchronize(ctx->stream));
+    int n = 0;
+    for (auto &pr : ctx->prof_events) {
+        float t = 0.f;
+        CK(cudaEventElapsedTime(&t, pr.first, pr.second));
+        if (n < cap) ms[n] = t;
+        n++;
+        cudaEventDestroy(pr.first); cudaEventDestroy(pr.second);
+    }
+    *n_launches = n;
+    ctx->prof_events.clear();
+    return TSAR_OK;
+}
+
 int tsar_dbg_candidate_stats(tsar_ctx *ctx, int colour, unsigned long long *out) {
     int rc = need_ready(ctx);
     if (rc) return rc;
@@ -1202,6 +1233,12 @@ int tsar_dbg_candidate_stats(tsar_ctx *ctx, int colour, unsigned long long *out)
 int tsar_dbg_eval_rounding(tsar_ctx *ctx, int wrapper_rounding) {
     if (!ctx) return TSAR_ERR_ARG;
     ctx->eval_wrapper_rounding = wrapper_rounding ? 1 : 0;
+    return TSAR_OK;
+}
+
+int tsar_dbg_quad_sampling(tsar_ctx *ctx, int checker_launches) {
+    if (!ctx) return TSAR_ERR_ARG;
+    ctx->quad_launches = checker_launches < 0 ? -1 : checker_launches;
     return TSAR_OK;
 }
 

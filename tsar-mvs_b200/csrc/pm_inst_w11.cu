@@ -16,4 +16,5 @@
 #endif
 #define PM_N1 6
 #define PM_GEN false
+#define PM_QUAD 1   // quad-cooperative sampling kernels (pm_core.cuh, view_cost_quad)
 #include "pm_inst.inc"

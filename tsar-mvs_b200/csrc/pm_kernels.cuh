@@ -31,6 +31,18 @@ struct WinSmem {
     }
 };
 
+// quad sampling scratch (QuadScratch) of the thread's warp, behind the window table (quad_smem_offset)
+template <int NT, int N1>
+__device__ __forceinline__ QuadScratch<N1 ? N1 : 2> quad_scratch(unsigned char *base, int tid) {
+    using QS = QuadScratch<N1 ? N1 : 2>;
+    unsigned char *w = base + quad_smem_offset(NT, N1 * N1) + (size_t)(tid >> 5) * QS::bytes_per_warp();
+    QS q;
+    q.h = reinterpret_cast<float4 *>(w);
+    q.n = reinterpret_cast<uint16_t *>(w + 32 * kQuadHWords * sizeof(float4));
+    q.lane = tid & 31;
+    return q;
+}
+
 template <int N1>
 __device__ __forceinline__ void fill_spatial_table(const PmConst &c, float *sp, int tid, int nthreads) {
     const int n1y = N1 ? N1 : c.n1y;
@@ -45,7 +57,7 @@ __device__ __forceinline__ void fill_spatial_table(const PmConst &c, float *sp, 
 // ---------------------------------------------------------------------------------------------
 // (1) random plane initialisation -- gipuma_init_cu2 (gipuma.cu:679-729)
 // ---------------------------------------------------------------------------------------------
-template <int NT, int MINB, int N1, bool GEN, bool U8>
+template <int NT, int MINB, int N1, bool GEN, bool U8, bool QUAD>
 __global__ void __launch_bounds__(NT, MINB) pm_init_kernel(const __grid_constant__ PmConst c, const float *__restrict__ ref,
                                                      const uint32_t *__restrict__ rng, int rng_len,
                                                      float4 *__restrict__ plane, float *__restrict__ cost) {
@@ -54,8 +66,13 @@ __global__ void __launch_bounds__(NT, MINB) pm_init_kernel(const __grid_constant
     const int tid = threadIdx.y * blockDim.x + threadIdx.x;
     fill_spatial_table<N1>(c, sm.sp, tid, NT);
     __syncthreads();
-    const int x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y * blockDim.y + threadIdx.y;
-    if (x >= c.W || y >= c.H) return;
+    int x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y * blockDim.y + threadIdx.y;
+    const bool inside = x < c.W && y < c.H;
+    if (QUAD ? __all_sync(0xffffffffu, !inside) : !inside) return;
+    // quad sampling: a lane outside the image stays as a helper that fetches for its quad-mates; it works on the
+    // nearest pixel (every read in bounds) and stores nothing
+    if (QUAD) { x = min(x, c.W - 1); y = min(y, c.H - 1); }
+    const QuadScratch<N1 ? N1 : 2> qs = quad_scratch<NT, N1>(smem_raw, tid);
     const WPair<NT> wt{sm.wt + tid};
     const RefStats rs = window_weights<NT, N1>(c, ref, x, y, sm.sp, wt);
 
@@ -80,7 +97,8 @@ __global__ void __launch_bounds__(NT, MINB) pm_init_kernel(const __grid_constant
     const float depth = fdiv(fmul(c.f_cam0, c.baseline), disp);                  // :712
     float4 pl = make_float4(nx, ny, nz, 0.f);
     pl.w = plane_d(c, nx, ny, nz, x, y, depth);                                  // :715
-    const MvResult r = multiview_cost<NT, N1, GEN, false, U8>(c, x, y, pl, wt, rs);
+    const MvResult r = multiview_cost<NT, N1, GEN, false, U8, false, QUAD>(c, x, y, pl, wt, rs, inside, &qs);
+    if (QUAD && !inside) return;
     const size_t p = (size_t)y * c.W + x;
     plane[p] = pl;
     cost[p] = r.cost;
@@ -95,10 +113,11 @@ __global__ void __launch_bounds__(NT, MINB) pm_init_kernel(const __grid_constant
 // colours), the thread's own result goes to `*_out` (which may alias `*_in` when DO_SP is false).
 // ---------------------------------------------------------------------------------------------
 
-template <int NT, int MINB, int N1, bool GEN, bool U8, bool DO_SP, bool DO_PR, bool TILE, bool PIN>
+template <int NT, int MINB, int N1, bool GEN, bool U8, bool DO_SP, bool DO_PR, bool TILE, bool PIN, bool QUAD>
 __global__ void __launch_bounds__(NT, MINB) pm_checker_kernel(const __grid_constant__ PmConst c,
                                                         const float *__restrict__ ref, const CheckerArgs a) {
     static_assert(!TILE || N1 > 0, "the tile layout needs a compile-time window");
+    static_assert(!QUAD || (!TILE && PM_WARP_COLS == 32), "quad sampling: pair table, quads of 4 adjacent columns");
     extern __shared__ __align__(16) unsigned char smem_raw[];
     WinSmem<NT> sm(smem_raw, N1 ? N1 * N1 : c.ns);   // (TILE: the table holds floats, see checker_smem_bytes)
     const int tid = threadIdx.y * 32 + threadIdx.x;
@@ -122,10 +141,15 @@ __global__ void __launch_bounds__(NT, MINB) pm_checker_kernel(const __grid_const
     // block = 32 columns x (NT/32) row pairs; lane parity selects the row of the pair exactly as the reference's
     // wrappers do (gipuma.cu:1099-1103).  (More compact warp footprints, PM_WARP_COLS = 16 or 8, measure the same to 0.3 %: texture wavefronts are per quad.)
     constexpr int WC = PM_WARP_COLS, WPR = 32 / WC;   // warps side by side in the 32-column tile
-    const int x = blockIdx.x * 32 + ((int)threadIdx.y % WPR) * WC + ((int)threadIdx.x % WC);
+    int x = blockIdx.x * 32 + ((int)threadIdx.y % WPR) * WC + ((int)threadIdx.x % WC);
     const int rowpair = ((int)threadIdx.y / WPR) * (32 / WC) + ((int)threadIdx.x / WC);
-    const int y = (blockIdx.y * (NT / 32) + rowpair) * 2 + ((x + a.colour) & 1);
-    if (x >= W || y >= H || y >= c.y_limit) return;
+    int y = (blockIdx.y * (NT / 32) + rowpair) * 2 + ((x + a.colour) & 1);
+    const bool inside = x < W && y < H && y < c.y_limit;
+    if (QUAD ? __all_sync(0xffffffffu, !inside) : !inside) return;
+    // quad sampling: a lane outside the image or past y_limit stays as a helper that fetches for its quad-mates; it
+    // works on the nearest pixel of the image (every read in bounds), evaluates nothing and stores nothing
+    if (QUAD) { x = min(x, W - 1); y = min(y, H - 1); }
+    const QuadScratch<N1 ? N1 : 2> qs = quad_scratch<NT, N1>(smem_raw, tid);
     const int own = a.colour;
     const int pidx = y * W + x;
 
@@ -162,6 +186,7 @@ __global__ void __launch_bounds__(NT, MINB) pm_checker_kernel(const __grid_const
 #pragma unroll 1
     for (int step = DO_SP ? 0 : 8;; step++) {
         float4 cand;
+        if (QUAD) cand = norm_now;   // a lane that evaluates nothing still publishes a homography to its quad
         float cand_depth = 0.f;
         bool eval = false;
         if (step < 8) {
@@ -203,15 +228,17 @@ __global__ void __launch_bounds__(NT, MINB) pm_checker_kernel(const __grid_const
             deltaZ = fdiv(deltaZ, 10.0f);
             deltaN = fmul(deltaN, 0.25f);
         }
-        if (eval) {
-            const MvResult r = multiview_cost<NT, N1, GEN, false, U8, PIN>(c, x, y, cand, wt, rs);
-            if (r.cost < cost_now) {
+        if (QUAD) eval = eval && inside;
+        if (QUAD ? __any_sync(0xffffffffu, eval) : eval) {
+            const MvResult r = multiview_cost<NT, N1, GEN, false, U8, PIN, QUAD>(c, x, y, cand, wt, rs, eval, &qs);
+            if (eval && r.cost < cost_now) {
                 cost_now = r.cost; norm_now = cand; ratio_now = r.ratio; beview_now = r.beview; meta_dirty = true;
                 depth_now = cand_depth;  // only read by the refinement rounds
             }
         }
     }
 
+    if (QUAD && !inside) return;
     a.cost_out[pidx] = cost_now;
     a.plane_out[pidx] = norm_now;
     if (meta_dirty) { a.ratio[pidx] = ratio_now; a.beview[pidx] = beview_now; }

@@ -23,10 +23,14 @@ enum { PM_MODE_SP = 1, PM_MODE_PR = 2, PM_MODE_FUSED = 3 };
 
 struct PmVariant {
     const char *name;
+    // quad != 0 (only where has_quad; init: with u8, checker: with u8 and PmConst::k_pinhole): quad-cooperative
+    // sampling (pm_core.cuh, view_cost_quad); otherwise cudaErrorInvalidValue.  Bit-identical results.
+    bool has_quad;
     // u8 != 0: sample the 8-bit copies of the source views (PmConst::tex8); bit-identical results
-    cudaError_t (*init)(int u8, const PmConst &, const float *ref, const uint32_t *rng, int rng_len, float4 *plane,
-                        float *cost, cudaStream_t);
-    cudaError_t (*checker)(int u8, int mode, const PmConst &, const float *ref, const CheckerArgs &, cudaStream_t);
+    cudaError_t (*init)(int u8, int quad, const PmConst &, const float *ref, const uint32_t *rng, int rng_len,
+                        float4 *plane, float *cost, cudaStream_t);
+    cudaError_t (*checker)(int u8, int quad, int mode, const PmConst &, const float *ref, const CheckerArgs &,
+                           cudaStream_t);
     cudaError_t (*eval)(int u8, int wrapper_rounding, const PmConst &, const float *ref, int n, const int2 *xy, const float4 *planes, float *cost,
                         int *beview, float *ratio, cudaStream_t);
     cudaError_t (*cost_of_state)(int u8, const PmConst &, const float *ref, const float4 *plane, float *cost, cudaStream_t);

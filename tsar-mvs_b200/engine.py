@@ -259,6 +259,16 @@ class DepthmapEngine:
         self._ck(self.lib.tsar_profile_read(self.h, C.byref(ms), C.byref(n)), "tsar_profile_read")
         return ms.value, n.value
 
+    def profile_read_launches(self, cap=4096):
+        """CUDA-event ms of each checkerboard launch since profiling was enabled (consumes them, as profile_read)."""
+        ms, n = (C.c_float * cap)(), C.c_int(0)
+        self._ck(self.lib.tsar_profile_read_launches(self.h, ms, int(cap), C.byref(n)), "tsar_profile_read_launches")
+        return [ms[k] for k in range(min(n.value, cap))]
+
+    def quad_sampling(self, checker_launches):
+        """tsar_dbg_quad_sampling: < 0 off; >= 0 init and the first checker_launches checkerboard launches."""
+        self._ck(self.lib.tsar_dbg_quad_sampling(self.h, int(checker_launches)), "tsar_dbg_quad_sampling")
+
     def candidate_stats(self, colour):
         """Counters of the propagation candidates the checkerboard launch of `colour` would try on the current state
         (tsar_dbg_candidate_stats): dict of counts + histogram of distinct candidates per pixel."""
