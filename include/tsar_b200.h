@@ -312,6 +312,35 @@ const char *tsar_fusion_last_error(const tsar_fusion *f);
 /* Resolution rounds of the last run: the most any view needed and the sum over the views (data-dependent). */
 int tsar_fusion_dbg_rounds(const tsar_fusion *f, int *max_rounds, long long *total_rounds);
 
+/* ---- cloud-to-cloud evaluation (DESIGN.md section 4.7) ---------------------------------------------------------------
+ * Scores a reconstruction R (n points) against a ground truth G (m points), float32 xyz in one frame and unit.
+ * dist(q, P) = sqrt_rn(min over the finite p of P of (dx dx + dy dy) + dz dz, d = p - q, float32, one rounding per
+ * operation) when that root is <= tau_max, else +inf; +inf for a non-finite q or a P without finite points.
+ * within_R[i] = #{r in R : dist(r, G) <= thresholds[i]}, within_G[i] = #{g in G : dist(g, R) <= thresholds[i]}.
+ * Accuracy = within_R / n, completeness = within_G / m (tsar-mvs_b200/cloud_eval.py).  This is not the ETH3D or
+ * Tanks and Temples evaluator.  A handle of its own; its device scratch only grows, so a second run with clouds no
+ * larger than before allocates nothing.  Device memory: 56 B per point of each cloud plus about 2 B per point of tree
+ * and the radix-sort scratch. */
+#define TSAR_EVAL_MAX_THRESHOLDS 64
+
+typedef struct tsar_eval tsar_eval;
+
+/* `stream` as in tsar_create.  TSAR_ERR_NODEVICE without an sm_100 device. */
+int tsar_eval_create(int device, void *stream, tsar_eval **out);
+/* Host pointers: recon = n_recon * 3 floats, gt = n_gt * 3 floats (either count may be 0; at most 2^31 - 1 each),
+ * thresholds = 1..64 finite values > 0, none above tau_max (finite, > 0).  within_recon / within_gt receive
+ * n_thresholds counts each.  dist_recon (n_recon floats) / dist_gt (n_gt floats) receive the per-point distances in
+ * input order; NULL = not wanted.  TSAR_ERR_ARG on bad sizes, pointers or thresholds, TSAR_ERR_NOMEM when the clouds
+ * do not fit. */
+int tsar_eval_run(tsar_eval *e, const float *recon, long long n_recon, const float *gt, long long n_gt,
+                  const float *thresholds, int n_thresholds, float tau_max, long long *within_recon,
+                  long long *within_gt, float *dist_recon, float *dist_gt);
+int tsar_eval_destroy(tsar_eval *e);
+const char *tsar_eval_last_error(const tsar_eval *e);
+/* Tree leaves visited in the last run, per direction (0 = R against G, 1 = G against R): total over the queries and
+ * the most one query visited. */
+int tsar_eval_dbg_visits(const tsar_eval *e, long long total[2], int max_per_query[2]);
+
 #ifdef __cplusplus
 }
 #endif

@@ -8,6 +8,6 @@ task names it); import it through `__graft_entry__.load_package()` or importlib.
 from . import _lib  # noqa: F401
 from .engine import DepthmapEngine, TsarError, make_params  # noqa: F401
 from . import scene  # noqa: F401
-from . import dmb, shard, cli, texture, counts, fusion  # noqa: F401
+from . import dmb, shard, cli, texture, counts, fusion, cloud_eval  # noqa: F401
 
-__all__ = ["DepthmapEngine", "TsarError", "make_params", "scene", "dmb", "shard", "fusion"]
+__all__ = ["DepthmapEngine", "TsarError", "make_params", "scene", "dmb", "shard", "fusion", "cloud_eval"]

@@ -66,6 +66,7 @@ EXPORTS = [
     "tsar_weak_edges", "tsar_weak_connect", "tsar_weak_boundary", "tsar_weak_close_border", "tsar_weak_regions", "tsar_set_labels_quarter", "tsar_scale_from_weak_png", "tsar_scale_from_confidence", "tsar_download_outputs",
     "tsar_fusion_create", "tsar_fusion_set_view", "tsar_fusion_run", "tsar_fusion_points", "tsar_fusion_destroy",
     "tsar_fusion_last_error", "tsar_fusion_dbg_rounds",
+    "tsar_eval_create", "tsar_eval_run", "tsar_eval_destroy", "tsar_eval_last_error", "tsar_eval_dbg_visits",
 ]
 
 
@@ -143,6 +144,11 @@ def load():
         "tsar_fusion_destroy": (i, [vp]),
         "tsar_fusion_last_error": (C.c_char_p, [vp]),
         "tsar_fusion_dbg_rounds": (i, [vp, ip, C.POINTER(C.c_longlong)]),
+        "tsar_eval_create": (i, [i, vp, C.POINTER(vp)]),
+        "tsar_eval_run": (i, [vp, vp, C.c_longlong, vp, C.c_longlong, vp, i, C.c_float, vp, vp, vp, vp]),
+        "tsar_eval_destroy": (i, [vp]),
+        "tsar_eval_last_error": (C.c_char_p, [vp]),
+        "tsar_eval_dbg_visits": (i, [vp, vp, vp]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(lib, name)

@@ -24,6 +24,10 @@ tsar_fit_region_planes and are completed by update_scale(_2).  `-no_weak_texture
 `-fuse` fuses every view's `APD/<stem>/TSAR_disp.dmb` + `TSAR_normals.dmb` with the colour images, cams and pair.txt
 into one point cloud, `<mslp>/TSAR_fused.ply` (fusion.py, DESIGN.md section 4.6; one GPU, views in dataset order).
 With `-all_views` it runs after the last view (single process only: fusion reads every view's output).
+`-eval <gt.ply>` scores `<mslp>/TSAR_fused.ply` against a ground-truth cloud (cloud_eval.py, DESIGN.md section 4.7):
+accuracy, completeness and F-score per threshold (`-eval_thresholds 0.01,0.02,...`, scene units; default
+0.01,0.02,0.05,0.1,0.2,0.5), one table line each, and `<mslp>/TSAR_eval.json`.  It runs alone on an existing
+TSAR_fused.ply or after `-fuse` / `-all_views -fuse` in the same call.
 Extra: `--synthetic=<C1|C2|small|tiny>` first writes a synthetic dataset in the reference's folder layout.
 
 `-all_views` replaces the per-view process loop of the run scripts (scripts/pipes.sh:30-49): every image of the
@@ -35,6 +39,7 @@ output files are already complete (an interrupted run continues where it stopped
 name and renamed, so a partial file never counts).
 """
 import itertools
+import math
 import os
 import sys
 
@@ -47,7 +52,7 @@ NUMERIC = {"blocksize", "iterations", "n_best", "cost_gamma", "depth_min", "dept
            "cam_scale", "cost_tau_color", "cost_tau_gradient", "cost_alpha", "disp_tol", "normal_tol", "census_epsilon",
            "self_similarity_n", "good_factor", "num_img_processed", "seed", "synthetic", "device", "lanes", "io_threads"}
 PATHS = {"images_folder", "mslp_folder", "krt_file", "output_folder", "p_folder", "camera_folder", "calib_file", "pmvs_folder",
-         "bounding_folder", "regions_file", "regions_text", "regions_size"}
+         "bounding_folder", "regions_file", "regions_text", "regions_size", "eval", "eval_thresholds"}
 BOOLS = {"color_processing", "view_selection", "import_apd", "no_display", "all_views", "no_weak_texture", "write_ply", "wmf", "no_slic", "no_write", "resume", "fuse"}
 
 
@@ -56,7 +61,7 @@ def parse_args(argv):
     opt = dict(images=[], blocksize=19, iterations=8, n_best=2, cost_comb=1, cam_scale=1.0, depth_min=-1.0, depth_max=-1.0,
                seed=20240601, device=0, images_folder="", mslp_folder="", output_folder="", synthetic=None,
                color_processing=False, import_apd=False, all_views=False, no_weak_texture=False, write_ply=False, wmf=False, no_slic=False, no_write=False, resume=False, fuse=False,
-               regions_file=None, regions_text=None, regions_size=None, lanes=2, io_threads=4)
+               regions_file=None, regions_text=None, regions_size=None, lanes=2, io_threads=4, eval=None, eval_thresholds=None)
     i = 0
     while i < len(argv):
         a = argv[i]
@@ -283,12 +288,24 @@ def run(argv):
             print("[tsar_cli] -fuse runs on one GPU (view v depends on the views before it): run -all_views under several "
                   "ranks without -fuse, then `tsar_cli.py -fuse -mslp_folder ...` as a single process", file=sys.stderr)
             return 2
+        if opt["eval"] and int(os.environ.get("WORLD_SIZE", "1")) > 1:
+            print("[tsar_cli] -eval runs in a single process: run -all_views under several ranks without it, then "
+                  "`tsar_cli.py -fuse -eval <gt.ply> -mslp_folder ...`", file=sys.stderr)
+            return 2
         run_all_views(opt, mslp)
         if opt["fuse"]:
-            return run_fuse(opt, mslp)
+            rc = run_fuse(opt, mslp)
+            if rc or not opt["eval"]:
+                return rc
+        if opt["eval"]:
+            return run_eval(opt, mslp)
         return 0
     if opt["fuse"]:
-        return run_fuse(opt, mslp)
+        rc = run_fuse(opt, mslp)
+        if rc or not opt["eval"]:
+            return rc
+    if opt["eval"]:
+        return run_eval(opt, mslp)
     if not opt["images"]:
         print(__doc__)
         return 2
@@ -426,6 +443,56 @@ def run_fuse(opt, mslp, quiet=False):
     dmb.write_fused_ply(out, xyz, nrm, rgb)
     if not quiet:
         print(f"[tsar_cli] fused {n_views} views ({W}x{H}) into {len(xyz)} points in {time.perf_counter() - t0:.2f} s -> {out}")
+    return 0
+
+
+def parse_thresholds(text):
+    """-eval_thresholds: comma-separated finite values > 0.  Raises ValueError naming the bad item."""
+    from .cloud_eval import MAX_THRESHOLDS
+    items = [t.strip() for t in (text or "").split(",") if t.strip()]
+    if not items:
+        raise ValueError("-eval_thresholds: empty threshold list")
+    if len(items) > MAX_THRESHOLDS:
+        raise ValueError(f"-eval_thresholds: at most {MAX_THRESHOLDS} thresholds")
+    out = []
+    for t in items:
+        try:
+            v = float(t)
+        except ValueError:
+            v = math.nan
+        if not (math.isfinite(v) and v > 0 and math.isfinite(np.float32(v)) and np.float32(v) > 0):
+            raise ValueError(f"-eval_thresholds: bad threshold {t!r} (need finite values > 0)")
+        out.append(v)
+    return out
+
+
+def run_eval(opt, mslp, quiet=False):
+    """-eval: <mslp>/TSAR_fused.ply against the ground-truth cloud -> table + <mslp>/TSAR_eval.json.  Returns the exit
+    code."""
+    import json
+    from . import cloud_eval
+    from .engine import TsarError
+    recon_path, gt_path = os.path.join(mslp, "TSAR_fused.ply"), opt["eval"]
+    try:
+        thresholds = parse_thresholds(opt["eval_thresholds"]) if opt["eval_thresholds"] is not None \
+            else list(cloud_eval.DEFAULT_THRESHOLDS)
+        recon = dmb.read_ply_points(recon_path)
+        gt = dmb.read_ply_points(gt_path)
+        res = cloud_eval.evaluate(recon, gt, thresholds, device=int(opt["device"]))
+    except (ValueError, TsarError) as e:
+        print(f"[tsar_cli] -eval: {e}", file=sys.stderr)
+        return 1
+    if not quiet:
+        print(f"[tsar_cli] -eval {recon_path} ({res['n_recon']} points) against {gt_path} ({res['n_gt']} points)")
+        for i, t in enumerate(res["thresholds"]):
+            print(f"[tsar_cli]   tau {t:g}: accuracy {res['accuracy'][i]:.4f} ({res['within_recon'][i]}), completeness "
+                  f"{res['completeness'][i]:.4f} ({res['within_gt'][i]}), F {res['fscore'][i]:.4f}")
+    out = {k: v for k, v in res.items()}
+    for k in ("accuracy", "completeness", "fscore"):      # JSON has no NaN: an empty cloud's fractions are null
+        out[k] = [None if math.isnan(v) else v for v in out[k]]
+    out = dict(recon=os.path.abspath(recon_path), gt=os.path.abspath(gt_path), **out)
+    with open(os.path.join(mslp, "TSAR_eval.json"), "w") as f:
+        json.dump(out, f, indent=1)
     return 0
 
 

@@ -87,3 +87,77 @@ def read_model_ply(path):
                 break
         rec = np.fromfile(f, dtype=PLY_VERTEX, count=n)
     return rec["p"], rec["n"], rec["c"]
+
+
+PLY_SCALARS = {"char": "i1", "int8": "i1", "uchar": "u1", "uint8": "u1", "short": "i2", "int16": "i2", "ushort": "u2",
+               "uint16": "u2", "int": "i4", "int32": "i4", "uint": "u4", "uint32": "u4", "float": "f4", "float32": "f4",
+               "double": "f8", "float64": "f8"}
+
+
+def read_ply_points(path):
+    """xyz of the vertex element of a PLY file ([n][3] float32; double coordinates are rounded once).  Reads
+    binary_little_endian and ascii files with any scalar property types and any extra properties (TSAR_fused.ply and
+    typical ground-truth scans); elements before the vertex element are skipped when they have no list property.
+    Anything else raises a one-line ValueError naming the file and the reason."""
+    def fail(reason):
+        return ValueError(f"{path}: {reason}")
+    try:
+        f = open(path, "rb")
+    except OSError as e:
+        raise fail(f"cannot open ({e.strerror})") from None
+    with f:
+        if f.readline().strip() != b"ply":
+            raise fail("not a PLY file")
+        fmt, elements = None, []                     # elements: [name, count, [(name, dtype or None for a list)]]
+        while True:
+            raw = f.readline()
+            if not raw:
+                raise fail("header has no end_header")
+            tok = raw.decode("ascii", "replace").split()
+            if not tok or tok[0] in ("comment", "obj_info"):
+                continue
+            if tok[0] == "end_header":
+                break
+            if tok[0] == "format" and len(tok) >= 2:
+                fmt = tok[1]
+            elif tok[0] == "element" and len(tok) == 3:
+                elements.append([tok[1], int(tok[2]), []])
+            elif tok[0] == "property" and elements and len(tok) >= 3:
+                if tok[1] == "list":
+                    elements[-1][2].append((tok[-1], None))
+                elif tok[1] in PLY_SCALARS:
+                    elements[-1][2].append((tok[2], PLY_SCALARS[tok[1]]))
+                else:
+                    raise fail(f"unknown property type {tok[1]}")
+            else:
+                raise fail(f"malformed header line {raw.strip()[:60]!r}")
+        if fmt not in ("binary_little_endian", "ascii"):
+            raise fail(f"unsupported format {fmt} (binary_little_endian or ascii only)")
+        names = [e[0] for e in elements]
+        if "vertex" not in names:
+            raise fail("no vertex element")
+        k = names.index("vertex")
+        for e in elements[:k + 1]:
+            if any(dt is None for _, dt in e[2]):
+                raise fail(f"list property in element {e[0]} (cannot locate the vertices)")
+        props = [p for p, _ in elements[k][2]]
+        if not all(c in props for c in "xyz"):
+            raise fail("vertex element has no x, y, z properties")
+        n = elements[k][1]
+        if fmt == "ascii":
+            for e in elements[:k]:
+                for _ in range(e[1]):
+                    f.readline()
+            lines = [f.readline() for _ in range(n)]
+            try:
+                rows = np.array([ln.split() for ln in lines], np.float64).reshape(n, len(props))
+            except ValueError:
+                raise fail(f"vertex data is not {n} rows of {len(props)} numbers") from None
+            return np.stack([rows[:, props.index(c)] for c in "xyz"], -1).astype(np.float32)
+        for e in elements[:k]:
+            f.seek(e[1] * np.dtype([(p, "<" + dt) for p, dt in e[2]]).itemsize, 1)
+        dt = np.dtype([(p, "<" + t) for p, t in elements[k][2]])
+        rec = np.fromfile(f, dtype=dt, count=n)
+        if len(rec) != n:
+            raise fail(f"truncated vertex data ({len(rec)} of {n} vertices)")
+        return np.stack([rec[c] for c in "xyz"], -1).astype(np.float32)

@@ -126,6 +126,33 @@ def render_rig(cfg, seed=1234, backend="numpy", device=None, depth_range=(0.7, 1
         yield i, img
 
 
+def rig_ground_truth_points(cfg, stride, spacing, backend="numpy", device=None):
+    """The visible ground truth of a rig as a point cloud ([n][3] float32): every `stride`-th pixel (both axes) of the
+    rendered ground-truth depth of every view is back-projected in float64 (X = C + depth * R^T K^-1 (x, y, 1)), then
+    thinned to one point per voxel of size `spacing` (voxel = floor(X / spacing)): the first point in view order, then
+    raster order, is kept.  Deterministic.  The facets are not sampled directly because facet 0 is unbounded; what the
+    cameras see bounds it."""
+    K, Rs, Cs, _ = make_rig(cfg)
+    sc = Scene(cfg["W"], cfg["H"], cfg["fx"], cfg["radius"], seed=1234)
+    Kinv = np.linalg.inv(K)
+    ys, xs = np.mgrid[0:cfg["H"]:stride, 0:cfg["W"]:stride]
+    rays = np.stack([xs, ys, np.ones_like(xs)], -1).reshape(-1, 3).astype(np.float64) @ Kinv.T
+    pts = []
+    for R, C in zip(Rs, Cs):
+        cam = dict(K_inv=Kinv, _R_world=R, _C_world=C)
+        if backend == "torch":
+            depth = sc.render_torch(cam, cfg["W"], cfg["H"], device)[1].cpu().numpy().astype(np.float64)
+        else:
+            depth = sc.render(cam, cfg["W"], cfg["H"])[1]
+        d = depth[::stride, ::stride].reshape(-1)
+        ok = np.isfinite(d)
+        pts.append(C + d[ok, None] * (rays[ok] @ R))
+    X = np.concatenate(pts)
+    vox = np.floor(X / spacing).astype(np.int64)
+    _, first = np.unique(vox, axis=0, return_index=True)
+    return X[np.sort(first)].astype(np.float32)
+
+
 class Scene:
     """Piecewise-planar scene in world coordinates, sized to the reference camera's frustum."""
 
