@@ -32,7 +32,7 @@ typedef enum tsar_status {
     TSAR_ERR_ARG = -1,     /* bad argument (null, size, V outside [1,32], ...) */
     TSAR_ERR_STATE = -2,   /* call order (e.g. iterate before set_views)        */
     TSAR_ERR_CUDA = -3,    /* a CUDA runtime call failed                        */
-    TSAR_ERR_NOMEM = -4,
+    TSAR_ERR_NOMEM = -4,   /* a device or pinned allocation failed              */
     TSAR_ERR_NODEVICE = -5 /* no CUDA device / not an sm_100 part: there is no CPU fallback */
 } tsar_status;
 

@@ -22,9 +22,11 @@
 
 #include <algorithm>
 #include <cub/device/device_radix_sort.cuh>
+#include <memory>
 #include <string>
 
 #include "../../include/tsar_b200.h"
+#include "dev_mem.h"
 #include "pm_math.cuh"
 
 using namespace tsar;
@@ -282,12 +284,11 @@ __global__ void __launch_bounds__(kQueryThreads) eval_query_kernel(TreeArgs t, Q
 
 // Device buffers of one cloud; they only grow.
 struct CloudBuf {
-    long long cap = 0, node_cap = 0;
-    float *xyz = nullptr;
-    unsigned long long *key[2] = {nullptr, nullptr};
-    int *idx[2] = {nullptr, nullptr};
-    float4 *pts = nullptr, *lo = nullptr, *hi = nullptr;
-    float *dist = nullptr;
+    DeviceBuf<float> xyz;
+    DeviceBuf<unsigned long long> key[2];
+    DeviceBuf<int> idx[2];
+    DeviceBuf<float4> pts, lo, hi;
+    DeviceBuf<float> dist;
     // of the current run
     long long n = 0, n_finite = 0;
     int n_levels = 0;
@@ -306,58 +307,27 @@ struct Misc {
 
 }  // namespace
 
-struct tsar_eval {
-    int device = 0;
-    cudaStream_t stream = nullptr;
-    bool own_stream = false;
-    std::string err;
+struct tsar_eval : HandleCore {
     CloudBuf c[2];                  // 0 = reconstruction, 1 = ground truth
-    void *d_sort_tmp = nullptr;
-    size_t sort_tmp_cap = 0;
-    Misc *d_misc = nullptr, *h_misc = nullptr;
+    DeviceBuf<unsigned char> sort_tmp;
+    DeviceBuf<Misc> d_misc;
+    PinnedBuf<Misc> h_misc;
     long long visits_total[2] = {0, 0};
     int visits_max[2] = {0, 0};
 };
-
-#define ECK(call)                                                                                             \
-    do {                                                                                                      \
-        cudaError_t e_ = (call);                                                                              \
-        if (e_ != cudaSuccess) {                                                                              \
-            char buf_[512];                                                                                   \
-            snprintf(buf_, sizeof(buf_), "%s:%d %s: %s", __FILE__, __LINE__, #call, cudaGetErrorString(e_));  \
-            e->err = buf_;                                                                                    \
-            cudaGetLastError();                                                                               \
-            return e_ == cudaErrorMemoryAllocation ? TSAR_ERR_NOMEM : TSAR_ERR_CUDA;                          \
-        }                                                                                                     \
-    } while (0)
-
-#define EFAIL(code, msg) \
-    do {                 \
-        e->err = (msg);  \
-        return (code);   \
-    } while (0)
-
-static void cloud_free(CloudBuf &c) {
-    cudaFree(c.xyz); cudaFree(c.key[0]); cudaFree(c.key[1]); cudaFree(c.idx[0]); cudaFree(c.idx[1]);
-    cudaFree(c.pts); cudaFree(c.lo); cudaFree(c.hi); cudaFree(c.dist);
-    c = CloudBuf();
-}
 
 static unsigned blocks(long long n, int threads) { return (unsigned)((n + threads - 1) / threads); }
 
 // Capacity for n points: 12 (input) + 2 x 8 (keys) + 2 x 4 (indices) + 16 (sorted points) + 4 (distances) = 56 B each.
 static int cloud_reserve(tsar_eval *e, CloudBuf &c, long long n) {
-    if (n <= c.cap) return TSAR_OK;
-    cloud_free(c);
     const size_t N = (size_t)n;
-    ECK(cudaMalloc(&c.xyz, 3 * N * sizeof(float)));
-    ECK(cudaMalloc(&c.key[0], N * sizeof(unsigned long long)));
-    ECK(cudaMalloc(&c.key[1], N * sizeof(unsigned long long)));
-    ECK(cudaMalloc(&c.idx[0], N * sizeof(int)));
-    ECK(cudaMalloc(&c.idx[1], N * sizeof(int)));
-    ECK(cudaMalloc(&c.pts, N * sizeof(float4)));
-    ECK(cudaMalloc(&c.dist, N * sizeof(float)));
-    c.cap = n;
+    TSAR_CK(e, c.xyz.reserve(3 * N));
+    TSAR_CK(e, c.key[0].reserve(N));
+    TSAR_CK(e, c.key[1].reserve(N));
+    TSAR_CK(e, c.idx[0].reserve(N));
+    TSAR_CK(e, c.idx[1].reserve(N));
+    TSAR_CK(e, c.pts.reserve(N));
+    TSAR_CK(e, c.dist.reserve(N));
     return TSAR_OK;
 }
 
@@ -397,36 +367,11 @@ extern "C" {
 int tsar_eval_create(int device, void *stream, tsar_eval **out) {
     if (!out) return TSAR_ERR_ARG;
     *out = nullptr;
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0 || device < 0 || device >= ndev) {
-        cudaGetLastError();
-        fprintf(stderr, "[tsar_b200] no usable CUDA device (requested %d of %d); this library has no CPU path\n", device, ndev);
-        return TSAR_ERR_NODEVICE;
-    }
-    cudaDeviceProp prop;
-    if (cudaGetDeviceProperties(&prop, device) != cudaSuccess || prop.major != 10) {
-        fprintf(stderr, "[tsar_b200] device %d is sm_%d%d; this build contains sm_100a code only\n", device, prop.major, prop.minor);
-        return TSAR_ERR_NODEVICE;
-    }
-    if (cudaSetDevice(device) != cudaSuccess) return TSAR_ERR_CUDA;
-    tsar_eval *e = new tsar_eval;
-    e->device = device;
-    bool ok = true;
-    if (stream) e->stream = (cudaStream_t)stream;
-    else {
-        ok = cudaStreamCreateWithFlags(&e->stream, cudaStreamNonBlocking) == cudaSuccess;
-        e->own_stream = ok;
-    }
-    ok = ok && cudaMalloc(&e->d_misc, sizeof(Misc)) == cudaSuccess && cudaMallocHost(&e->h_misc, sizeof(Misc)) == cudaSuccess;
-    if (!ok) {
-        cudaGetLastError();
-        cudaFree(e->d_misc);
-        cudaFreeHost(e->h_misc);
-        if (e->own_stream) cudaStreamDestroy(e->stream);
-        delete e;
-        return TSAR_ERR_NOMEM;
-    }
-    *out = e;
+    std::unique_ptr<tsar_eval> e(new tsar_eval);
+    if (int rc = e->open(device, stream)) return rc;
+    TSAR_CK(e, e->d_misc.reserve(1));
+    TSAR_CK(e, e->h_misc.reserve(1));
+    *out = e.release();
     return TSAR_OK;
 }
 
@@ -434,12 +379,6 @@ int tsar_eval_destroy(tsar_eval *e) {
     if (!e) return TSAR_OK;
     cudaSetDevice(e->device);
     cudaStreamSynchronize(e->stream);
-    cloud_free(e->c[0]);
-    cloud_free(e->c[1]);
-    cudaFree(e->d_sort_tmp);
-    cudaFree(e->d_misc);
-    cudaFreeHost(e->h_misc);
-    if (e->own_stream) cudaStreamDestroy(e->stream);
     delete e;
     return TSAR_OK;
 }
@@ -451,24 +390,24 @@ int tsar_eval_run(tsar_eval *e, const float *recon, long long n_recon, const flo
                   long long *within_gt, float *dist_recon, float *dist_gt) {
     if (!e) return TSAR_ERR_ARG;
     if (n_recon < 0 || n_gt < 0 || n_recon > kMaxPoints || n_gt > kMaxPoints)
-        EFAIL(TSAR_ERR_ARG, "tsar_eval_run: point counts must lie in 0 .. 2^31 - 1");
-    if ((n_recon && !recon) || (n_gt && !gt)) EFAIL(TSAR_ERR_ARG, "tsar_eval_run: null cloud");
+        TSAR_FAIL(e, TSAR_ERR_ARG, "tsar_eval_run: point counts must lie in 0 .. 2^31 - 1");
+    if ((n_recon && !recon) || (n_gt && !gt)) TSAR_FAIL(e, TSAR_ERR_ARG, "tsar_eval_run: null cloud");
     if (n_thresholds < 1 || n_thresholds > TSAR_EVAL_MAX_THRESHOLDS)
-        EFAIL(TSAR_ERR_ARG, "tsar_eval_run: 1..64 thresholds");
-    if (!thresholds || !within_recon || !within_gt) EFAIL(TSAR_ERR_ARG, "tsar_eval_run: null thresholds or counts");
+        TSAR_FAIL(e, TSAR_ERR_ARG, "tsar_eval_run: 1..64 thresholds");
+    if (!thresholds || !within_recon || !within_gt) TSAR_FAIL(e, TSAR_ERR_ARG, "tsar_eval_run: null thresholds or counts");
     if (!(tau_max > 0.0f) || !(tau_max <= 3.402823466e38f))
-        EFAIL(TSAR_ERR_ARG, "tsar_eval_run: tau_max must be finite and > 0");
+        TSAR_FAIL(e, TSAR_ERR_ARG, "tsar_eval_run: tau_max must be finite and > 0");
     QueryArgs qa{};
     qa.k = n_thresholds;
     qa.tau_max = tau_max;
     qa.cut2 = cut_square(tau_max);
     for (int i = 0; i < n_thresholds; ++i) {
         const float t = thresholds[i];
-        if (!(t > 0.0f) || !(t <= 3.402823466e38f)) EFAIL(TSAR_ERR_ARG, "tsar_eval_run: thresholds must be finite and > 0");
-        if (t > tau_max) EFAIL(TSAR_ERR_ARG, "tsar_eval_run: a threshold exceeds tau_max");
+        if (!(t > 0.0f) || !(t <= 3.402823466e38f)) TSAR_FAIL(e, TSAR_ERR_ARG, "tsar_eval_run: thresholds must be finite and > 0");
+        if (t > tau_max) TSAR_FAIL(e, TSAR_ERR_ARG, "tsar_eval_run: a threshold exceeds tau_max");
         qa.tau[i] = t;
     }
-    ECK(cudaSetDevice(e->device));
+    TSAR_CK(e, cudaSetDevice(e->device));
     const float *host[2] = {recon, gt};
     const long long n[2] = {n_recon, n_gt};
     size_t tmp_need = 0;
@@ -477,97 +416,85 @@ int tsar_eval_run(tsar_eval *e, const float *recon, long long n_recon, const flo
         if (rc != TSAR_OK) return rc;
         size_t bytes = 0;
         if (n[c]) {
-            ECK(cub::DeviceRadixSort::SortPairs(nullptr, bytes, e->c[c].key[0], e->c[c].key[1], e->c[c].idx[0],
-                                                e->c[c].idx[1], (int)n[c], 0, 64, e->stream));
+            TSAR_CK(e, cub::DeviceRadixSort::SortPairs(nullptr, bytes, e->c[c].key[0].get(), e->c[c].key[1].get(), e->c[c].idx[0].get(),
+                                                e->c[c].idx[1].get(), (int)n[c], 0, 64, e->stream));
         }
         tmp_need = std::max(tmp_need, bytes);
     }
-    if (tmp_need > e->sort_tmp_cap) {
-        cudaFree(e->d_sort_tmp);
-        e->d_sort_tmp = nullptr;
-        e->sort_tmp_cap = 0;
-        ECK(cudaMalloc(&e->d_sort_tmp, tmp_need));
-        e->sort_tmp_cap = tmp_need;
-    }
+    TSAR_CK(e, e->sort_tmp.reserve(tmp_need));
     Misc init{};
     for (int c = 0; c < 2; ++c)
         for (int a = 0; a < 3; ++a) {
             init.box[c][a] = 0xffffffffu;
             init.box[c][3 + a] = 0u;
         }
-    *e->h_misc = init;
-    ECK(cudaMemcpyAsync(e->d_misc, e->h_misc, sizeof(Misc), cudaMemcpyHostToDevice, e->stream));
+    *e->h_misc.get() = init;
+    TSAR_CK(e, cudaMemcpyAsync(e->d_misc.get(), e->h_misc.get(), sizeof(Misc), cudaMemcpyHostToDevice, e->stream));
     for (int c = 0; c < 2; ++c) {
         CloudBuf &b = e->c[c];
         b.n = n[c];
         if (!n[c]) continue;
-        ECK(cudaMemcpyAsync(b.xyz, host[c], 3 * (size_t)n[c] * sizeof(float), cudaMemcpyHostToDevice, e->stream));
+        TSAR_CK(e, cudaMemcpyAsync(b.xyz.get(), host[c], 3 * (size_t)n[c] * sizeof(float), cudaMemcpyHostToDevice, e->stream));
         eval_bbox_kernel<<<std::min(blocks(n[c], kThreads), 148u * 8u), kThreads, 0, e->stream>>>(
-            b.xyz, n[c], e->d_misc->box[c], &e->d_misc->n_finite[c]);
-        eval_key_kernel<<<blocks(n[c], kThreads), kThreads, 0, e->stream>>>(b.xyz, n[c], e->d_misc->box[c], b.key[0], b.idx[0]);
-        ECK(cudaGetLastError());
-        size_t bytes = e->sort_tmp_cap;
-        ECK(cub::DeviceRadixSort::SortPairs(e->d_sort_tmp, bytes, b.key[0], b.key[1], b.idx[0], b.idx[1], (int)n[c], 0, 64,
+            b.xyz.get(), n[c], e->d_misc.get()->box[c], &e->d_misc.get()->n_finite[c]);
+        eval_key_kernel<<<blocks(n[c], kThreads), kThreads, 0, e->stream>>>(b.xyz.get(), n[c], e->d_misc.get()->box[c], b.key[0].get(), b.idx[0].get());
+        TSAR_CK(e, cudaGetLastError());
+        size_t bytes = e->sort_tmp.capacity();
+        TSAR_CK(e, cub::DeviceRadixSort::SortPairs(e->sort_tmp.get(), bytes, b.key[0].get(), b.key[1].get(), b.idx[0].get(), b.idx[1].get(), (int)n[c], 0, 64,
                                             e->stream));
-        eval_gather_kernel<<<blocks(n[c], kThreads), kThreads, 0, e->stream>>>(b.xyz, n[c], b.idx[1], b.pts);
-        ECK(cudaGetLastError());
+        eval_gather_kernel<<<blocks(n[c], kThreads), kThreads, 0, e->stream>>>(b.xyz.get(), n[c], b.idx[1].get(), b.pts.get());
+        TSAR_CK(e, cudaGetLastError());
     }
-    ECK(cudaMemcpyAsync(e->h_misc, e->d_misc, sizeof(Misc), cudaMemcpyDeviceToHost, e->stream));
-    ECK(cudaStreamSynchronize(e->stream));
+    TSAR_CK(e, cudaMemcpyAsync(e->h_misc.get(), e->d_misc.get(), sizeof(Misc), cudaMemcpyDeviceToHost, e->stream));
+    TSAR_CK(e, cudaStreamSynchronize(e->stream));
     for (int c = 0; c < 2; ++c) {
         CloudBuf &b = e->c[c];
-        b.n_finite = (long long)e->h_misc->n_finite[c];
+        b.n_finite = (long long)e->h_misc.get()->n_finite[c];
         tree_shape(b);
         const long long nodes = tree_nodes(b);
-        if (nodes > b.node_cap) {
-            cudaFree(b.lo); cudaFree(b.hi);
-            b.lo = b.hi = nullptr;
-            b.node_cap = 0;
-            ECK(cudaMalloc(&b.lo, (size_t)nodes * sizeof(float4)));
-            ECK(cudaMalloc(&b.hi, (size_t)nodes * sizeof(float4)));
-            b.node_cap = nodes;
-        }
+        TSAR_CK(e, b.lo.reserve((size_t)nodes));
+        TSAR_CK(e, b.hi.reserve((size_t)nodes));
         if (!b.n_levels) continue;
-        eval_leaf_kernel<<<blocks(b.len[0], kThreads), kThreads, 0, e->stream>>>(b.pts, b.n_finite, b.len[0], b.lo, b.hi);
+        eval_leaf_kernel<<<blocks(b.len[0], kThreads), kThreads, 0, e->stream>>>(b.pts.get(), b.n_finite, b.len[0], b.lo.get(), b.hi.get());
         for (int l = 1; l < b.n_levels; ++l)
             eval_merge_kernel<<<blocks(b.len[l], kThreads), kThreads, 0, e->stream>>>(
-                b.lo + b.off[l - 1], b.hi + b.off[l - 1], b.len[l - 1], b.len[l], b.lo + b.off[l], b.hi + b.off[l]);
-        ECK(cudaGetLastError());
+                b.lo.get() + b.off[l - 1], b.hi.get() + b.off[l - 1], b.len[l - 1], b.len[l], b.lo.get() + b.off[l], b.hi.get() + b.off[l]);
+        TSAR_CK(e, cudaGetLastError());
     }
     // direction 0: reconstruction points against the ground-truth index; direction 1: the reverse
     for (int dir = 0; dir < 2; ++dir) {
         const CloudBuf &q = e->c[dir], &ix = e->c[1 - dir];
         if (!q.n) continue;
         TreeArgs ta{};
-        ta.pts = ix.pts;
-        ta.lo = ix.lo;
-        ta.hi = ix.hi;
+        ta.pts = ix.pts.get();
+        ta.lo = ix.lo.get();
+        ta.hi = ix.hi.get();
         ta.n_finite = ix.n_finite;
         ta.n_levels = ix.n_levels;
         for (int l = 0; l < ix.n_levels; ++l) {
             ta.off[l] = ix.off[l];
             ta.len[l] = ix.len[l];
         }
-        qa.q = q.pts;
-        qa.q_idx = q.idx[1];
+        qa.q = q.pts.get();
+        qa.q_idx = q.idx[1].get();
         qa.n = q.n;
         eval_query_kernel<<<blocks(q.n, kQueryThreads), kQueryThreads, 0, e->stream>>>(
-            ta, qa, q.dist, e->d_misc->within[dir], &e->d_misc->visits_total[dir], &e->d_misc->visits_max[dir]);
-        ECK(cudaGetLastError());
+            ta, qa, q.dist.get(), e->d_misc.get()->within[dir], &e->d_misc.get()->visits_total[dir], &e->d_misc.get()->visits_max[dir]);
+        TSAR_CK(e, cudaGetLastError());
     }
-    ECK(cudaMemcpyAsync(e->h_misc, e->d_misc, sizeof(Misc), cudaMemcpyDeviceToHost, e->stream));
+    TSAR_CK(e, cudaMemcpyAsync(e->h_misc.get(), e->d_misc.get(), sizeof(Misc), cudaMemcpyDeviceToHost, e->stream));
     float *dist_out[2] = {dist_recon, dist_gt};
     for (int c = 0; c < 2; ++c)
         if (dist_out[c] && n[c])
-            ECK(cudaMemcpyAsync(dist_out[c], e->c[c].dist, (size_t)n[c] * sizeof(float), cudaMemcpyDeviceToHost, e->stream));
-    ECK(cudaStreamSynchronize(e->stream));
+            TSAR_CK(e, cudaMemcpyAsync(dist_out[c], e->c[c].dist.get(), (size_t)n[c] * sizeof(float), cudaMemcpyDeviceToHost, e->stream));
+    TSAR_CK(e, cudaStreamSynchronize(e->stream));
     for (int i = 0; i < n_thresholds; ++i) {
-        within_recon[i] = (long long)e->h_misc->within[0][i];
-        within_gt[i] = (long long)e->h_misc->within[1][i];
+        within_recon[i] = (long long)e->h_misc.get()->within[0][i];
+        within_gt[i] = (long long)e->h_misc.get()->within[1][i];
     }
     for (int d = 0; d < 2; ++d) {
-        e->visits_total[d] = (long long)e->h_misc->visits_total[d];
-        e->visits_max[d] = (int)e->h_misc->visits_max[d];
+        e->visits_total[d] = (long long)e->h_misc.get()->visits_total[d];
+        e->visits_max[d] = (int)e->h_misc.get()->visits_max[d];
     }
     return TSAR_OK;
 }

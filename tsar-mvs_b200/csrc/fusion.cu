@@ -19,10 +19,12 @@
 #include <string.h>
 
 #include <algorithm>
+#include <memory>
 #include <string>
 #include <vector>
 
 #include "../../include/tsar_b200.h"
+#include "dev_mem.h"
 #include "pm_math.cuh"
 
 using namespace tsar;
@@ -264,61 +266,32 @@ __global__ void __launch_bounds__(kThreads) fusion_emit_kernel(ViewArgs a, const
 
 }  // namespace
 
-struct tsar_fusion {
-    int device = 0;
-    cudaStream_t stream = nullptr;
-    bool own_stream = false;
-    std::string err;
+struct tsar_fusion : HandleCore {
     int n_views = 0, W = 0, H = 0;
     size_t P = 0;
     std::vector<FusionCam> cams;
     std::vector<std::vector<int>> neighbours;  // empty = view not set
     // resident inputs: 21 B per pixel and view
-    FusionCam *d_cams = nullptr;
-    float4 *d_dn = nullptr;
-    uchar4 *d_col = nullptr;
-    unsigned char *d_mask = nullptr;
+    DeviceBuf<FusionCam> d_cams;
+    DeviceBuf<float4> d_dn;
+    DeviceBuf<uchar4> d_col;
+    DeviceBuf<unsigned char> d_mask;
     // scratch for one view
-    int *d_cand = nullptr, *d_owner = nullptr;
-    int scratch_src = 0;  // neighbours the cand / owner buffers hold
-    unsigned char *d_state[2] = {nullptr, nullptr};
-    int *d_block = nullptr, *d_counters = nullptr;  // block counts + offsets; counters = {undecided, total}
-    float *d_xyz = nullptr, *d_nrm = nullptr;
-    unsigned char *d_rgb = nullptr;
+    DeviceBuf<int> d_cand, d_owner;
+    DeviceBuf<unsigned char> d_state[2];
+    DeviceBuf<int> d_block, d_counters;  // block counts + offsets; counters = {undecided, total}
+    DeviceBuf<float> d_xyz, d_nrm;
+    DeviceBuf<unsigned char> d_rgb;
     // pinned landing buffers of one view, and the points of the last run
-    float *h_xyz = nullptr, *h_nrm = nullptr;
-    unsigned char *h_rgb = nullptr;
-    int *h_counters = nullptr;
+    PinnedBuf<float> h_xyz, h_nrm;
+    PinnedBuf<unsigned char> h_rgb;
+    PinnedBuf<int> h_counters;
     std::vector<float> xyz, nrm;
     std::vector<unsigned char> rgb;
     long long n_points = 0;
     int rounds_max = 0;
     long long rounds_total = 0;
 };
-
-#define FCK(call)                                                                                   \
-    do {                                                                                            \
-        cudaError_t e_ = (call);                                                                    \
-        if (e_ != cudaSuccess) {                                                                    \
-            char buf_[512];                                                                         \
-            snprintf(buf_, sizeof(buf_), "%s:%d %s: %s", __FILE__, __LINE__, #call, cudaGetErrorString(e_)); \
-            f->err = buf_;                                                                          \
-            return TSAR_ERR_CUDA;                                                                   \
-        }                                                                                           \
-    } while (0)
-
-#define FFAIL(code, msg)   \
-    do {                   \
-        f->err = (msg);    \
-        return (code);     \
-    } while (0)
-
-static void fusion_free(tsar_fusion *f) {
-    cudaFree(f->d_cams); cudaFree(f->d_dn); cudaFree(f->d_col); cudaFree(f->d_mask);
-    cudaFree(f->d_cand); cudaFree(f->d_owner); cudaFree(f->d_state[0]); cudaFree(f->d_state[1]);
-    cudaFree(f->d_block); cudaFree(f->d_counters); cudaFree(f->d_xyz); cudaFree(f->d_nrm); cudaFree(f->d_rgb);
-    cudaFreeHost(f->h_xyz); cudaFreeHost(f->h_nrm); cudaFreeHost(f->h_rgb); cudaFreeHost(f->h_counters);
-}
 
 // K^-1 by the adjugate in double, rounded once to float (oc_fuse computes it the same way).
 static bool invert3(const float *K, float *out) {
@@ -340,19 +313,8 @@ int tsar_fusion_create(int device, void *stream, int n_views, int W, int H, tsar
     *out = nullptr;
     // pixel indices are int: the last block's p must not overflow, and no index may reach the owner sentinel 0x7f7f7f7f
     if (n_views < 1 || W < 1 || H < 1 || (long long)W * H > 0x7f7f7f7fLL - kThreads) return TSAR_ERR_ARG;
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0 || device < 0 || device >= ndev) {
-        fprintf(stderr, "[tsar_b200] no usable CUDA device (requested %d of %d); this library has no CPU path\n", device, ndev);
-        return TSAR_ERR_NODEVICE;
-    }
-    cudaDeviceProp prop;
-    if (cudaGetDeviceProperties(&prop, device) != cudaSuccess || prop.major != 10) {
-        fprintf(stderr, "[tsar_b200] device %d is sm_%d%d; this build contains sm_100a code only\n", device, prop.major, prop.minor);
-        return TSAR_ERR_NODEVICE;
-    }
-    if (cudaSetDevice(device) != cudaSuccess) return TSAR_ERR_CUDA;
-    tsar_fusion *f = new tsar_fusion;
-    f->device = device;
+    std::unique_ptr<tsar_fusion> f(new tsar_fusion);
+    if (int rc = f->open(device, stream)) return rc;
     f->n_views = n_views;
     f->W = W;
     f->H = H;
@@ -360,31 +322,22 @@ int tsar_fusion_create(int device, void *stream, int n_views, int W, int H, tsar
     f->cams.resize(n_views);
     f->neighbours.resize(n_views);
     const size_t P = f->P, N = (size_t)n_views, nb = (P + kThreads - 1) / kThreads;
-    bool ok = true;
-    if (stream) f->stream = (cudaStream_t)stream;
-    else {
-        ok = cudaStreamCreateWithFlags(&f->stream, cudaStreamNonBlocking) == cudaSuccess;
-        f->own_stream = ok;
-    }
-    ok = ok && cudaMalloc(&f->d_cams, N * sizeof(FusionCam)) == cudaSuccess &&
-         cudaMalloc(&f->d_dn, N * P * sizeof(float4)) == cudaSuccess &&
-         cudaMalloc(&f->d_col, N * P * sizeof(uchar4)) == cudaSuccess && cudaMalloc(&f->d_mask, N * P) == cudaSuccess &&
-         cudaMalloc(&f->d_state[0], P) == cudaSuccess && cudaMalloc(&f->d_state[1], P) == cudaSuccess &&
-         cudaMalloc(&f->d_block, 2 * nb * sizeof(int)) == cudaSuccess &&
-         cudaMalloc(&f->d_counters, 2 * sizeof(int)) == cudaSuccess &&
-         cudaMalloc(&f->d_xyz, 3 * P * sizeof(float)) == cudaSuccess &&
-         cudaMalloc(&f->d_nrm, 3 * P * sizeof(float)) == cudaSuccess && cudaMalloc(&f->d_rgb, 3 * P) == cudaSuccess &&
-         cudaMallocHost(&f->h_xyz, 3 * P * sizeof(float)) == cudaSuccess &&
-         cudaMallocHost(&f->h_nrm, 3 * P * sizeof(float)) == cudaSuccess && cudaMallocHost(&f->h_rgb, 3 * P) == cudaSuccess &&
-         cudaMallocHost(&f->h_counters, 2 * sizeof(int)) == cudaSuccess;
-    if (!ok) {
-        cudaGetLastError();
-        fusion_free(f);
-        if (f->own_stream) cudaStreamDestroy(f->stream);
-        delete f;
-        return TSAR_ERR_NOMEM;
-    }
-    *out = f;
+    TSAR_CK(f, f->d_cams.reserve(N));
+    TSAR_CK(f, f->d_dn.reserve(N * P));
+    TSAR_CK(f, f->d_col.reserve(N * P));
+    TSAR_CK(f, f->d_mask.reserve(N * P));
+    TSAR_CK(f, f->d_state[0].reserve(P));
+    TSAR_CK(f, f->d_state[1].reserve(P));
+    TSAR_CK(f, f->d_block.reserve(2 * nb));
+    TSAR_CK(f, f->d_counters.reserve(2));
+    TSAR_CK(f, f->d_xyz.reserve(3 * P));
+    TSAR_CK(f, f->d_nrm.reserve(3 * P));
+    TSAR_CK(f, f->d_rgb.reserve(3 * P));
+    TSAR_CK(f, f->h_xyz.reserve(3 * P));
+    TSAR_CK(f, f->h_nrm.reserve(3 * P));
+    TSAR_CK(f, f->h_rgb.reserve(3 * P));
+    TSAR_CK(f, f->h_counters.reserve(2));
+    *out = f.release();
     return TSAR_OK;
 }
 
@@ -392,8 +345,6 @@ int tsar_fusion_destroy(tsar_fusion *f) {
     if (!f) return TSAR_OK;
     cudaSetDevice(f->device);
     cudaStreamSynchronize(f->stream);
-    fusion_free(f);
-    if (f->own_stream) cudaStreamDestroy(f->stream);
     delete f;
     return TSAR_OK;
 }
@@ -403,34 +354,34 @@ const char *tsar_fusion_last_error(const tsar_fusion *f) { return f ? f->err.c_s
 int tsar_fusion_set_view(tsar_fusion *f, int view, const tsar_view_camera *cam, const float *depth, const float *normals,
                          const unsigned char *bgr, const int *neighbours, int n_neighbours) {
     if (!f) return TSAR_ERR_ARG;
-    if (view < 0 || view >= f->n_views) FFAIL(TSAR_ERR_ARG, "tsar_fusion_set_view: view index out of range");
-    if (!cam || !depth || !normals || !bgr || !neighbours) FFAIL(TSAR_ERR_ARG, "tsar_fusion_set_view: null pointer");
+    if (view < 0 || view >= f->n_views) TSAR_FAIL(f, TSAR_ERR_ARG, "tsar_fusion_set_view: view index out of range");
+    if (!cam || !depth || !normals || !bgr || !neighbours) TSAR_FAIL(f, TSAR_ERR_ARG, "tsar_fusion_set_view: null pointer");
     if (n_neighbours < 1 || n_neighbours > TSAR_FUSION_MAX_NEIGHBOURS)
-        FFAIL(TSAR_ERR_ARG, "tsar_fusion_set_view: a view needs 1..32 neighbours");
+        TSAR_FAIL(f, TSAR_ERR_ARG, "tsar_fusion_set_view: a view needs 1..32 neighbours");
     std::vector<int> nb(neighbours, neighbours + n_neighbours);
     for (int j = 0; j < n_neighbours; ++j) {
-        if (nb[j] < 0 || nb[j] >= f->n_views) FFAIL(TSAR_ERR_ARG, "tsar_fusion_set_view: neighbour index out of range");
-        if (nb[j] == view) FFAIL(TSAR_ERR_ARG, "tsar_fusion_set_view: a view cannot be its own neighbour");
+        if (nb[j] < 0 || nb[j] >= f->n_views) TSAR_FAIL(f, TSAR_ERR_ARG, "tsar_fusion_set_view: neighbour index out of range");
+        if (nb[j] == view) TSAR_FAIL(f, TSAR_ERR_ARG, "tsar_fusion_set_view: a view cannot be its own neighbour");
         for (int i = 0; i < j; ++i)
-            if (nb[i] == nb[j]) FFAIL(TSAR_ERR_ARG, "tsar_fusion_set_view: repeated neighbour");
+            if (nb[i] == nb[j]) TSAR_FAIL(f, TSAR_ERR_ARG, "tsar_fusion_set_view: repeated neighbour");
     }
     FusionCam c;
     memcpy(c.K, cam->K, sizeof c.K);
     memcpy(c.R, cam->R, sizeof c.R);
     memcpy(c.t, cam->t, sizeof c.t);
-    if (!invert3(c.K, c.Kinv)) FFAIL(TSAR_ERR_ARG, "tsar_fusion_set_view: K is singular");
-    FCK(cudaSetDevice(f->device));
+    if (!invert3(c.K, c.Kinv)) TSAR_FAIL(f, TSAR_ERR_ARG, "tsar_fusion_set_view: K is singular");
+    TSAR_CK(f, cudaSetDevice(f->device));
     const size_t P = f->P, vo = (size_t)view * P;
     // the host arrays land in the per-view output buffers (16 + 3 of their 27 bytes per pixel), then are packed
-    float *st_depth = f->d_xyz, *st_normals = f->d_nrm;
-    FCK(cudaMemcpyAsync(st_depth, depth, P * sizeof(float), cudaMemcpyHostToDevice, f->stream));
-    FCK(cudaMemcpyAsync(st_normals, normals, 3 * P * sizeof(float), cudaMemcpyHostToDevice, f->stream));
-    FCK(cudaMemcpyAsync(f->d_rgb, bgr, 3 * P, cudaMemcpyHostToDevice, f->stream));
+    float *st_depth = f->d_xyz.get(), *st_normals = f->d_nrm.get();
+    TSAR_CK(f, cudaMemcpyAsync(st_depth, depth, P * sizeof(float), cudaMemcpyHostToDevice, f->stream));
+    TSAR_CK(f, cudaMemcpyAsync(st_normals, normals, 3 * P * sizeof(float), cudaMemcpyHostToDevice, f->stream));
+    TSAR_CK(f, cudaMemcpyAsync(f->d_rgb.get(), bgr, 3 * P, cudaMemcpyHostToDevice, f->stream));
     fusion_pack_kernel<<<(unsigned)((P + kThreads - 1) / kThreads), kThreads, 0, f->stream>>>(
-        st_depth, st_normals, f->d_rgb, P, f->d_dn + vo, f->d_col + vo);
-    FCK(cudaGetLastError());
-    FCK(cudaMemcpyAsync(f->d_cams + view, &c, sizeof c, cudaMemcpyHostToDevice, f->stream));
-    FCK(cudaStreamSynchronize(f->stream));
+        st_depth, st_normals, f->d_rgb.get(), P, f->d_dn.get() + vo, f->d_col.get() + vo);
+    TSAR_CK(f, cudaGetLastError());
+    TSAR_CK(f, cudaMemcpyAsync(f->d_cams.get() + view, &c, sizeof c, cudaMemcpyHostToDevice, f->stream));
+    TSAR_CK(f, cudaStreamSynchronize(f->stream));
     f->cams[view] = c;
     f->neighbours[view] = nb;
     return TSAR_OK;
@@ -438,30 +389,24 @@ int tsar_fusion_set_view(tsar_fusion *f, int view, const tsar_view_camera *cam, 
 
 int tsar_fusion_run(tsar_fusion *f, const tsar_fusion_params *prm, long long *n_points) {
     if (!f) return TSAR_ERR_ARG;
-    if (!prm) FFAIL(TSAR_ERR_ARG, "tsar_fusion_run: null parameters");
+    if (!prm) TSAR_FAIL(f, TSAR_ERR_ARG, "tsar_fusion_run: null parameters");
     if (!(prm->max_reproj_px > 0.0f) || !(prm->max_rel_depth > 0.0f) || !(prm->max_normal_deg >= 0.0f) ||
         !(prm->max_normal_deg <= 180.0f) || prm->min_consistent < 1)
-        FFAIL(TSAR_ERR_ARG, "tsar_fusion_run: parameters out of range (max_reproj_px > 0, max_rel_depth > 0, "
+        TSAR_FAIL(f, TSAR_ERR_ARG, "tsar_fusion_run: parameters out of range (max_reproj_px > 0, max_rel_depth > 0, "
                             "0 <= max_normal_deg <= 180, min_consistent >= 1)");
     int max_src = 0;
     for (int v = 0; v < f->n_views; ++v) {
         if (f->neighbours[v].empty()) {
             char buf[128];
             snprintf(buf, sizeof buf, "tsar_fusion_run: view %d was not set", v);
-            FFAIL(TSAR_ERR_ARG, buf);
+            TSAR_FAIL(f, TSAR_ERR_ARG, buf);
         }
         max_src = std::max(max_src, (int)f->neighbours[v].size());
     }
-    FCK(cudaSetDevice(f->device));
+    TSAR_CK(f, cudaSetDevice(f->device));
     const size_t P = f->P;
-    if (max_src > f->scratch_src) {
-        cudaFree(f->d_cand); cudaFree(f->d_owner);
-        f->d_cand = f->d_owner = nullptr;
-        f->scratch_src = 0;
-        FCK(cudaMalloc(&f->d_cand, (size_t)max_src * P * sizeof(int)));
-        FCK(cudaMalloc(&f->d_owner, (size_t)max_src * P * sizeof(int)));
-        f->scratch_src = max_src;
-    }
+    TSAR_CK(f, f->d_cand.reserve((size_t)max_src * P));
+    TSAR_CK(f, f->d_owner.reserve((size_t)max_src * P));
     const double kPi = 3.14159265358979323846;
     ViewArgs a{};
     a.W = f->W;
@@ -471,8 +416,8 @@ int tsar_fusion_run(tsar_fusion *f, const tsar_fusion_params *prm, long long *n_
     a.max_rel = prm->max_rel_depth;
     a.cos_normal = (float)cos((double)prm->max_normal_deg * (kPi / 180.0));
     const unsigned nb = (unsigned)((P + kThreads - 1) / kThreads);
-    int *d_block_count = f->d_block, *d_block_off = f->d_block + nb;
-    FCK(cudaMemsetAsync(f->d_mask, 0, (size_t)f->n_views * P, f->stream));
+    int *d_block_count = f->d_block.get(), *d_block_off = f->d_block.get() + nb;
+    TSAR_CK(f, cudaMemsetAsync(f->d_mask.get(), 0, (size_t)f->n_views * P, f->stream));
     f->xyz.clear(); f->nrm.clear(); f->rgb.clear();
     f->n_points = 0;
     f->rounds_max = 0;
@@ -482,41 +427,41 @@ int tsar_fusion_run(tsar_fusion *f, const tsar_fusion_params *prm, long long *n_
         a.v = v;
         a.n_src = (int)S.size();
         for (int j = 0; j < a.n_src; ++j) a.src[j] = S[j];
-        fusion_candidates_kernel<<<nb, kThreads, 0, f->stream>>>(a, f->d_cams, f->d_dn, f->d_mask, f->d_cand, f->d_state[0]);
-        FCK(cudaGetLastError());
+        fusion_candidates_kernel<<<nb, kThreads, 0, f->stream>>>(a, f->d_cams.get(), f->d_dn.get(), f->d_mask.get(), f->d_cand.get(), f->d_state[0].get());
+        TSAR_CK(f, cudaGetLastError());
         int cur = 0, rounds = 0;
         for (;;) {
-            FCK(cudaMemsetAsync(f->d_owner, 0x7f,   // 0x7f7f7f7f: no owner (larger than any pixel index)
+            TSAR_CK(f, cudaMemsetAsync(f->d_owner.get(), 0x7f,   // 0x7f7f7f7f: no owner (larger than any pixel index)
                                  (size_t)a.n_src * P * sizeof(int), f->stream));
-            FCK(cudaMemsetAsync(f->d_counters, 0, sizeof(int), f->stream));
-            fusion_claim_kernel<<<nb, kThreads, 0, f->stream>>>(a.n_src, (int)P, f->d_cand, f->d_state[cur], f->d_owner);
-            fusion_decide_kernel<<<nb, kThreads, 0, f->stream>>>(a.n_src, (int)P, a.min_consistent, f->d_cand, f->d_owner,
-                                                                 f->d_state[cur], f->d_state[cur ^ 1], f->d_counters);
-            FCK(cudaGetLastError());
-            FCK(cudaMemcpyAsync(f->h_counters, f->d_counters, sizeof(int), cudaMemcpyDeviceToHost, f->stream));
-            FCK(cudaStreamSynchronize(f->stream));
+            TSAR_CK(f, cudaMemsetAsync(f->d_counters.get(), 0, sizeof(int), f->stream));
+            fusion_claim_kernel<<<nb, kThreads, 0, f->stream>>>(a.n_src, (int)P, f->d_cand.get(), f->d_state[cur].get(), f->d_owner.get());
+            fusion_decide_kernel<<<nb, kThreads, 0, f->stream>>>(a.n_src, (int)P, a.min_consistent, f->d_cand.get(), f->d_owner.get(),
+                                                                 f->d_state[cur].get(), f->d_state[cur ^ 1].get(), f->d_counters.get());
+            TSAR_CK(f, cudaGetLastError());
+            TSAR_CK(f, cudaMemcpyAsync(f->h_counters.get(), f->d_counters.get(), sizeof(int), cudaMemcpyDeviceToHost, f->stream));
+            TSAR_CK(f, cudaStreamSynchronize(f->stream));
             cur ^= 1;
             ++rounds;
-            if (f->h_counters[0] == 0) break;
+            if (f->h_counters.get()[0] == 0) break;
         }
         f->rounds_max = std::max(f->rounds_max, rounds);
         f->rounds_total += rounds;
-        fusion_count_kernel<<<nb, kThreads, 0, f->stream>>>((int)P, f->d_state[cur], d_block_count);
-        fusion_scan_kernel<<<1, 1024, 0, f->stream>>>(d_block_count, (int)nb, d_block_off, f->d_counters + 1);
-        fusion_emit_kernel<<<nb, kThreads, 0, f->stream>>>(a, f->d_cams, f->d_dn, f->d_col, f->d_mask, f->d_cand, f->d_owner,
-                                                           f->d_state[cur], d_block_off, f->d_xyz, f->d_nrm, f->d_rgb);
-        FCK(cudaGetLastError());
-        FCK(cudaMemcpyAsync(f->h_counters + 1, f->d_counters + 1, sizeof(int), cudaMemcpyDeviceToHost, f->stream));
-        FCK(cudaStreamSynchronize(f->stream));
-        const size_t n = (size_t)f->h_counters[1];
+        fusion_count_kernel<<<nb, kThreads, 0, f->stream>>>((int)P, f->d_state[cur].get(), d_block_count);
+        fusion_scan_kernel<<<1, 1024, 0, f->stream>>>(d_block_count, (int)nb, d_block_off, f->d_counters.get() + 1);
+        fusion_emit_kernel<<<nb, kThreads, 0, f->stream>>>(a, f->d_cams.get(), f->d_dn.get(), f->d_col.get(), f->d_mask.get(), f->d_cand.get(), f->d_owner.get(),
+                                                           f->d_state[cur].get(), d_block_off, f->d_xyz.get(), f->d_nrm.get(), f->d_rgb.get());
+        TSAR_CK(f, cudaGetLastError());
+        TSAR_CK(f, cudaMemcpyAsync(f->h_counters.get() + 1, f->d_counters.get() + 1, sizeof(int), cudaMemcpyDeviceToHost, f->stream));
+        TSAR_CK(f, cudaStreamSynchronize(f->stream));
+        const size_t n = (size_t)f->h_counters.get()[1];
         if (n) {
-            FCK(cudaMemcpyAsync(f->h_xyz, f->d_xyz, 3 * n * sizeof(float), cudaMemcpyDeviceToHost, f->stream));
-            FCK(cudaMemcpyAsync(f->h_nrm, f->d_nrm, 3 * n * sizeof(float), cudaMemcpyDeviceToHost, f->stream));
-            FCK(cudaMemcpyAsync(f->h_rgb, f->d_rgb, 3 * n, cudaMemcpyDeviceToHost, f->stream));
-            FCK(cudaStreamSynchronize(f->stream));
-            f->xyz.insert(f->xyz.end(), f->h_xyz, f->h_xyz + 3 * n);
-            f->nrm.insert(f->nrm.end(), f->h_nrm, f->h_nrm + 3 * n);
-            f->rgb.insert(f->rgb.end(), f->h_rgb, f->h_rgb + 3 * n);
+            TSAR_CK(f, cudaMemcpyAsync(f->h_xyz.get(), f->d_xyz.get(), 3 * n * sizeof(float), cudaMemcpyDeviceToHost, f->stream));
+            TSAR_CK(f, cudaMemcpyAsync(f->h_nrm.get(), f->d_nrm.get(), 3 * n * sizeof(float), cudaMemcpyDeviceToHost, f->stream));
+            TSAR_CK(f, cudaMemcpyAsync(f->h_rgb.get(), f->d_rgb.get(), 3 * n, cudaMemcpyDeviceToHost, f->stream));
+            TSAR_CK(f, cudaStreamSynchronize(f->stream));
+            f->xyz.insert(f->xyz.end(), f->h_xyz.get(), f->h_xyz.get() + 3 * n);
+            f->nrm.insert(f->nrm.end(), f->h_nrm.get(), f->h_nrm.get() + 3 * n);
+            f->rgb.insert(f->rgb.end(), f->h_rgb.get(), f->h_rgb.get() + 3 * n);
             f->n_points += (long long)n;
         }
     }
@@ -526,9 +471,9 @@ int tsar_fusion_run(tsar_fusion *f, const tsar_fusion_params *prm, long long *n_
 
 int tsar_fusion_points(tsar_fusion *f, float *xyz, float *normals, unsigned char *rgb, long long capacity) {
     if (!f) return TSAR_ERR_ARG;
-    if (capacity < f->n_points) FFAIL(TSAR_ERR_ARG, "tsar_fusion_points: capacity is smaller than the number of points");
+    if (capacity < f->n_points) TSAR_FAIL(f, TSAR_ERR_ARG, "tsar_fusion_points: capacity is smaller than the number of points");
     const size_t n = (size_t)f->n_points;
-    if (n && (!xyz || !normals || !rgb)) FFAIL(TSAR_ERR_ARG, "tsar_fusion_points: null pointer");
+    if (n && (!xyz || !normals || !rgb)) TSAR_FAIL(f, TSAR_ERR_ARG, "tsar_fusion_points: null pointer");
     if (n) {
         memcpy(xyz, f->xyz.data(), 3 * n * sizeof(float));
         memcpy(normals, f->nrm.data(), 3 * n * sizeof(float));

@@ -17,6 +17,7 @@
 #include <cuda_runtime.h>
 
 #include "../../include/tsar_b200.h"
+#include "dev_mem.h"
 #include "pm_math.cuh"
 
 namespace tsar {
@@ -29,18 +30,12 @@ struct SpixelInfo {  // the fields of gSLICr::objects::spixel_info (gSLICr_spixe
 };
 
 struct SlicState {
-    int cap_px = 0, cap_sp = 0;
     int last_nsp = 0;       // superpixels of the last run (debug read-back)
-    uchar4 *d_in = nullptr;
-    float4 *d_lab = nullptr;
-    int *d_idx = nullptr, *d_tmp = nullptr;
-    SpixelInfo *d_sp = nullptr;
+    DeviceBuf<uchar4> d_in;
+    DeviceBuf<float4> d_lab;
+    DeviceBuf<int> d_idx, d_tmp;
+    DeviceBuf<SpixelInfo> d_sp;
 };
-
-static inline void slic_free(SlicState &s) {
-    cudaFree(s.d_in); cudaFree(s.d_lab); cudaFree(s.d_idx); cudaFree(s.d_tmp); cudaFree(s.d_sp);
-    s = SlicState();
-}
 
 // rgb2CIELab (gSLICr_seg_engine_shared.h:30-59); fusion pattern of the reference build: first product
 // rounded, the next two fused on top, divisions by the white point IEEE, L = fma(116, fy, -16)
@@ -211,52 +206,50 @@ __global__ void slic_enforce_kernel(const int *__restrict__ in, int *__restrict_
     out[y * w + x] = diff >= 16 ? dl : c;
 }
 
-// seg_engine::Perform_Segmentation (gSLICr_seg_engine.cpp:30-46) + Get_Seg_Mask.  Returns NULL or an error text.
-static inline const char *slic_run(SlicState &st, const unsigned char *bgrx, const tsar_slic_settings &cfg, int *labels_out,
-                                   cudaStream_t stream, int *n_launches) {
+// seg_engine::Perform_Segmentation (gSLICr_seg_engine.cpp:30-46) + Get_Seg_Mask.  Returns a tsar_status; the message of a
+// failure goes to hc.err.
+static inline int slic_run(HandleCore &hc, SlicState &st, const unsigned char *bgrx, const tsar_slic_settings &cfg,
+                           int *labels_out, cudaStream_t stream, int *n_launches) {
     *n_launches = 0;
     const int w = cfg.img_w, h = cfg.img_h, size = cfg.spixel_size;
-    if (w <= 0 || h <= 0 || size <= 0 || cfg.no_iters < 0) return "tsar_slic: bad settings";
+    if (w <= 0 || h <= 0 || size <= 0 || cfg.no_iters < 0) TSAR_FAIL(&hc, TSAR_ERR_CUDA, "tsar_slic: bad settings");
     const int mw = w / size, mh = h / size;  // (int)ceil(int/int): the division truncates first (GPU.cu:74-75)
-    if (mw < 1 || mh < 1) return "tsar_slic: image smaller than one superpixel";
+    if (mw < 1 || mh < 1) TSAR_FAIL(&hc, TSAR_ERR_CUDA, "tsar_slic: image smaller than one superpixel");
     const int npx = w * h, nsp = mw * mh;
     st.last_nsp = nsp;
-    if (npx > st.cap_px || nsp > st.cap_sp) {
-        slic_free(st);
-        if (cudaMalloc(&st.d_in, (size_t)npx * 4) || cudaMalloc(&st.d_lab, (size_t)npx * 16) || cudaMalloc(&st.d_idx, (size_t)npx * 4) ||
-            cudaMalloc(&st.d_tmp, (size_t)npx * 4) || cudaMalloc(&st.d_sp, (size_t)nsp * sizeof(SpixelInfo)))
-            return "tsar_slic: cudaMalloc failed";
-        st.cap_px = npx; st.cap_sp = nsp;
-        st.last_nsp = nsp;
-    }
+    TSAR_CK(&hc, st.d_in.reserve(npx));
+    TSAR_CK(&hc, st.d_lab.reserve(npx));
+    TSAR_CK(&hc, st.d_idx.reserve(npx));
+    TSAR_CK(&hc, st.d_tmp.reserve(npx));
+    TSAR_CK(&hc, st.d_sp.reserve(nsp));
     const int nblocks = (int)ceilf((float)(size * size * 9) / 256.0f);  // no_grid_per_center (GPU.cu:80-82)
     const int nbpl = size * 3 / 16;                                     // no_blocks_per_line (GPU.cu:160)
-    if (nbpl < 1) return "tsar_slic: spixel_size below 6 is not supported by the reference's block tiling";
+    if (nbpl < 1) TSAR_FAIL(&hc, TSAR_ERR_CUDA, "tsar_slic: spixel_size below 6 is not supported by the reference's block tiling");
     const float norm_xy = 1.0f / size;                                  // max_xy_dist (GPU.cu:88)
-    if (cudaMemcpyAsync(st.d_in, bgrx, (size_t)npx * 4, cudaMemcpyHostToDevice, stream)) return "tsar_slic: H2D failed";
-    cudaMemsetAsync(st.d_idx, 0, (size_t)npx * 4, stream);
+    if (cudaMemcpyAsync(st.d_in.get(), bgrx, (size_t)npx * 4, cudaMemcpyHostToDevice, stream)) TSAR_FAIL(&hc, TSAR_ERR_CUDA, "tsar_slic: H2D failed");
+    cudaMemsetAsync(st.d_idx.get(), 0, (size_t)npx * 4, stream);
     dim3 b(16, 16), gp((w + 15) / 16, (h + 15) / 16), gm((mw + 15) / 16, (mh + 15) / 16);
-    slic_cvt_lab_kernel<<<gp, b, 0, stream>>>(st.d_in, st.d_lab, w, h);
-    slic_init_centers_kernel<<<gm, b, 0, stream>>>(st.d_lab, st.d_sp, mw, mh, w, h, size);
-    slic_assign_kernel<<<gp, b, 0, stream>>>(st.d_lab, st.d_sp, st.d_idx, mw, mh, w, h, size, cfg.coh_weight, norm_xy);
+    slic_cvt_lab_kernel<<<gp, b, 0, stream>>>(st.d_in.get(), st.d_lab.get(), w, h);
+    slic_init_centers_kernel<<<gm, b, 0, stream>>>(st.d_lab.get(), st.d_sp.get(), mw, mh, w, h, size);
+    slic_assign_kernel<<<gp, b, 0, stream>>>(st.d_lab.get(), st.d_sp.get(), st.d_idx.get(), mw, mh, w, h, size, cfg.coh_weight, norm_xy);
     *n_launches += 3;
     for (int it = 0; it < cfg.no_iters; it++) {
         if (cfg.correct_reduction)
-            slic_update_full_kernel<<<(nsp * 32 + 127) / 128, 128, 0, stream>>>(st.d_lab, st.d_idx, st.d_sp, mw, mh, w, h, size);
+            slic_update_full_kernel<<<(nsp * 32 + 127) / 128, 128, 0, stream>>>(st.d_lab.get(), st.d_idx.get(), st.d_sp.get(), mw, mh, w, h, size);
         else
-            slic_update_parity_kernel<<<(nsp * 32 + 127) / 128, 128, 0, stream>>>(st.d_lab, st.d_idx, st.d_sp, mw, mh, w, h, size, nblocks, nbpl);
-        slic_assign_kernel<<<gp, b, 0, stream>>>(st.d_lab, st.d_sp, st.d_idx, mw, mh, w, h, size, cfg.coh_weight, norm_xy);
+            slic_update_parity_kernel<<<(nsp * 32 + 127) / 128, 128, 0, stream>>>(st.d_lab.get(), st.d_idx.get(), st.d_sp.get(), mw, mh, w, h, size, nblocks, nbpl);
+        slic_assign_kernel<<<gp, b, 0, stream>>>(st.d_lab.get(), st.d_sp.get(), st.d_idx.get(), mw, mh, w, h, size, cfg.coh_weight, norm_xy);
         *n_launches += 2;
     }
     if (cfg.do_enforce_connectivity) {
-        slic_enforce_kernel<<<gp, b, 0, stream>>>(st.d_idx, st.d_tmp, w, h);
-        slic_enforce_kernel<<<gp, b, 0, stream>>>(st.d_tmp, st.d_idx, w, h);
+        slic_enforce_kernel<<<gp, b, 0, stream>>>(st.d_idx.get(), st.d_tmp.get(), w, h);
+        slic_enforce_kernel<<<gp, b, 0, stream>>>(st.d_tmp.get(), st.d_idx.get(), w, h);
         *n_launches += 2;
     }
-    if (cudaGetLastError() != cudaSuccess) return "tsar_slic: kernel launch failed";
-    if (cudaMemcpyAsync(labels_out, st.d_idx, (size_t)npx * 4, cudaMemcpyDeviceToHost, stream)) return "tsar_slic: D2H failed";
-    if (cudaStreamSynchronize(stream) != cudaSuccess) return "tsar_slic: execution failed";
-    return nullptr;
+    if (cudaGetLastError() != cudaSuccess) TSAR_FAIL(&hc, TSAR_ERR_CUDA, "tsar_slic: kernel launch failed");
+    if (cudaMemcpyAsync(labels_out, st.d_idx.get(), (size_t)npx * 4, cudaMemcpyDeviceToHost, stream)) TSAR_FAIL(&hc, TSAR_ERR_CUDA, "tsar_slic: D2H failed");
+    if (cudaStreamSynchronize(stream) != cudaSuccess) TSAR_FAIL(&hc, TSAR_ERR_CUDA, "tsar_slic: execution failed");
+    return TSAR_OK;
 }
 
 }  // namespace tsar
