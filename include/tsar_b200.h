@@ -341,6 +341,52 @@ const char *tsar_eval_last_error(const tsar_eval *e);
  * the most one query visited. */
 int tsar_eval_dbg_visits(const tsar_eval *e, long long total[2], int max_per_query[2]);
 
+/* ---- mesh extraction (DESIGN.md section 4.8) ---------------------------------------------------------------------------
+ * Integrates the per-view depth maps of a dataset into a truncated signed distance field on a dense voxel grid and
+ * extracts a coloured triangle mesh from it by marching tetrahedra on the Freudenthal split of every cell.  Grid point
+ * (i, j, k) sits at origin + ((float)i + 0.5f, ...) * voxel; its linear index is (k ny + j) nx + i.  Per point the views
+ * are visited in index order: a view whose depth D at the rounded projection is valid and has sdf = D - z >= -trunc adds
+ * fminf(1, sdf / trunc) to S and 1 to W; when also sdf <= trunc it adds the pixel's colour and 1 to Wc.  A point is
+ * defined when W >= min_weight (F = S / W) and inside when F < 0.  Only cells with 8 defined corners emit triangles; the
+ * right-hand normal of a triangle points from inside to outside.  Vertices are ordered by owning lattice point, then by
+ * edge direction 100, 010, 001, 110, 101, 011, 111; triangles by cell, tetrahedron, triangle.  Float32, one rounding per
+ * operation, so the result is identical to the sequential rule (oracle/mesh_cpu.c).  A handle of its own, all views of
+ * one W x H.  Device memory: 8 B per pixel and view, 20 B per grid point (S, W | Wc, three colour sums) plus 18 B per
+ * grid point of extraction scratch, plus the mesh (15 B per vertex, 12 B per triangle); every buffer only grows. */
+typedef struct tsar_mesh_grid { float origin[3]; float voxel; int dims[3]; } tsar_mesh_grid;
+typedef struct tsar_mesh_params {
+    float trunc;      /* truncation distance in scene units, finite and > 0 */
+    int min_weight;   /* views a grid point needs to be defined, 1..65535 */
+} tsar_mesh_params;
+typedef struct tsar_mesh tsar_mesh;
+
+/* `stream` as in tsar_create.  TSAR_ERR_ARG unless 1 <= n_views <= 65535 (W and Wc are u16) and W, H >= 1;
+ * TSAR_ERR_NODEVICE without an sm_100 device, TSAR_ERR_NOMEM when the views do not fit. */
+int tsar_mesh_create(int device, void *stream, int n_views, int W, int H, tsar_mesh **out);
+/* Host pointers: depth = W*H floats (camera z; a pixel is used when its depth is finite and > 0), bgr = W*H*3 bytes. */
+int tsar_mesh_set_view(tsar_mesh *m, int view, const tsar_view_camera *cam, const float *depth, const unsigned char *bgr);
+/* Integrates every view (all must be set) on the grid and extracts the mesh; it stays on the device until tsar_mesh_get.
+ * TSAR_ERR_ARG for a non-finite origin, a voxel or trunc that is not finite and > 0, a dimension outside [2, 2^23], more
+ * than 2^31 - 1 grid points or min_weight outside [1, 65535]; TSAR_ERR_NOMEM when the grid or the mesh does not fit
+ * (including more than 2^31 - 1 vertices). */
+int tsar_mesh_run(tsar_mesh *m, const tsar_mesh_grid *g, const tsar_mesh_params *p, long long *n_vertices,
+                  long long *n_triangles);
+/* The mesh of the last run: xyz 3 floats and rgb 3 bytes per vertex, 3 int32 vertex indices per triangle;
+ * TSAR_ERR_ARG when a capacity is smaller than the mesh. */
+int tsar_mesh_get(tsar_mesh *m, float *xyz, unsigned char *rgb, long long vertex_capacity, int *triangles,
+                  long long triangle_capacity);
+int tsar_mesh_destroy(tsar_mesh *m);
+const char *tsar_mesh_last_error(const tsar_mesh *m);
+/* Test-only.  dbg_extract: extract with the same kernels from a caller-supplied field of nx*ny*nz points (F, W, Wc and
+ * bgr_sum = 3 sums B, G, R per point; a defined point with F < 0 must have Wc >= 1, as integration guarantees), then
+ * tsar_mesh_get.  dbg_field: the field of the last tsar_mesh_run (F = S / W where W >= 1, else 0). */
+int tsar_mesh_dbg_extract(tsar_mesh *m, const tsar_mesh_grid *g, int min_weight, const float *F, const uint16_t *W,
+                          const uint16_t *Wc, const uint32_t *bgr_sum, long long *n_vertices, long long *n_triangles);
+int tsar_mesh_dbg_field(tsar_mesh *m, float *F, uint16_t *W, uint16_t *Wc, uint32_t *bgr_sum);
+/* CUDA-event times of the last completed tsar_mesh_run on the handle's stream: integration (the one kernel) and
+ * extraction (cells, vertex masks, scans, the host read of the totals, vertices, triangles). */
+int tsar_mesh_dbg_times(tsar_mesh *m, float *integrate_ms, float *extract_ms);
+
 #ifdef __cplusplus
 }
 #endif

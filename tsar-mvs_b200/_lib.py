@@ -51,6 +51,16 @@ class TsarFusionParams(C.Structure):
                 ("min_consistent", C.c_int)]
 
 
+class TsarMeshGrid(C.Structure):
+    """tsar_mesh_grid (DESIGN.md section 4.8): grid point (i, j, k) at origin + ((float)i + 0.5f, ...) * voxel."""
+    _fields_ = [("origin", C.c_float * 3), ("voxel", C.c_float), ("dims", C.c_int * 3)]
+
+
+class TsarMeshParams(C.Structure):
+    """tsar_mesh_params (DESIGN.md section 4.8)."""
+    _fields_ = [("trunc", C.c_float), ("min_weight", C.c_int)]
+
+
 # tsar_field
 F_NORM4, F_COST, F_DEPTH, F_FAKEDEPTH, F_SCALE, F_CANNY, F_RATIO, F_BEVIEW, F_LRDIFF, F_CONFID, \
     F_REGION_TEXT, F_REGION_NORM4 = range(12)
@@ -67,6 +77,8 @@ EXPORTS = [
     "tsar_fusion_create", "tsar_fusion_set_view", "tsar_fusion_run", "tsar_fusion_points", "tsar_fusion_destroy",
     "tsar_fusion_last_error", "tsar_fusion_dbg_rounds",
     "tsar_eval_create", "tsar_eval_run", "tsar_eval_destroy", "tsar_eval_last_error", "tsar_eval_dbg_visits",
+    "tsar_mesh_create", "tsar_mesh_set_view", "tsar_mesh_run", "tsar_mesh_get", "tsar_mesh_destroy", "tsar_mesh_last_error",
+    "tsar_mesh_dbg_extract", "tsar_mesh_dbg_field", "tsar_mesh_dbg_times",
 ]
 
 
@@ -149,6 +161,17 @@ def load():
         "tsar_eval_destroy": (i, [vp]),
         "tsar_eval_last_error": (C.c_char_p, [vp]),
         "tsar_eval_dbg_visits": (i, [vp, vp, vp]),
+        "tsar_mesh_create": (i, [i, vp, i, i, i, C.POINTER(vp)]),
+        "tsar_mesh_set_view": (i, [vp, i, C.POINTER(TsarViewCamera), vp, vp]),
+        "tsar_mesh_run": (i, [vp, C.POINTER(TsarMeshGrid), C.POINTER(TsarMeshParams), C.POINTER(C.c_longlong),
+                              C.POINTER(C.c_longlong)]),
+        "tsar_mesh_get": (i, [vp, vp, vp, C.c_longlong, vp, C.c_longlong]),
+        "tsar_mesh_destroy": (i, [vp]),
+        "tsar_mesh_last_error": (C.c_char_p, [vp]),
+        "tsar_mesh_dbg_extract": (i, [vp, C.POINTER(TsarMeshGrid), i, vp, vp, vp, vp, C.POINTER(C.c_longlong),
+                                      C.POINTER(C.c_longlong)]),
+        "tsar_mesh_dbg_field": (i, [vp, vp, vp, vp, vp]),
+        "tsar_mesh_dbg_times": (i, [vp, fp, fp]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(lib, name)

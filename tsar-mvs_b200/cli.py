@@ -28,6 +28,11 @@ With `-all_views` it runs after the last view (single process only: fusion reads
 accuracy, completeness and F-score per threshold (`-eval_thresholds 0.01,0.02,...`, scene units; default
 0.01,0.02,0.05,0.1,0.2,0.5), one table line each, and `<mslp>/TSAR_eval.json`.  It runs alone on an existing
 TSAR_fused.ply or after `-fuse` / `-all_views -fuse` in the same call.
+`-mesh` integrates every view's `APD/<stem>/TSAR_disp.dmb` with the colour images and cams into a truncated signed
+distance field and writes its surface as a coloured triangle mesh, `<mslp>/TSAR_mesh.ply` (mesh.py, DESIGN.md section
+4.8; one GPU).  The grid covers what the views see (mesh.default_grid) unless `-mesh_bbox x0,y0,z0,x1,y1,z1` gives the
+box; `-mesh_voxel <s>`, `-mesh_trunc <t>` (default 4 voxels) and `-mesh_min_weight <k>` (default 3) set the rest.  It
+runs alone or after `-all_views` / `-fuse` in the same call, before `-eval` (which still scores TSAR_fused.ply).
 Extra: `--synthetic=<C1|C2|small|tiny>` first writes a synthetic dataset in the reference's folder layout.
 
 `-all_views` replaces the per-view process loop of the run scripts (scripts/pipes.sh:30-49): every image of the
@@ -52,8 +57,9 @@ NUMERIC = {"blocksize", "iterations", "n_best", "cost_gamma", "depth_min", "dept
            "cam_scale", "cost_tau_color", "cost_tau_gradient", "cost_alpha", "disp_tol", "normal_tol", "census_epsilon",
            "self_similarity_n", "good_factor", "num_img_processed", "seed", "synthetic", "device", "lanes", "io_threads"}
 PATHS = {"images_folder", "mslp_folder", "krt_file", "output_folder", "p_folder", "camera_folder", "calib_file", "pmvs_folder",
-         "bounding_folder", "regions_file", "regions_text", "regions_size", "eval", "eval_thresholds"}
-BOOLS = {"color_processing", "view_selection", "import_apd", "no_display", "all_views", "no_weak_texture", "write_ply", "wmf", "no_slic", "no_write", "resume", "fuse"}
+         "bounding_folder", "regions_file", "regions_text", "regions_size", "eval", "eval_thresholds",
+         "mesh_voxel", "mesh_bbox", "mesh_trunc", "mesh_min_weight"}
+BOOLS = {"color_processing", "view_selection", "import_apd", "no_display", "all_views", "no_weak_texture", "write_ply", "wmf", "no_slic", "no_write", "resume", "fuse", "mesh"}
 
 
 def parse_args(argv):
@@ -61,7 +67,8 @@ def parse_args(argv):
     opt = dict(images=[], blocksize=19, iterations=8, n_best=2, cost_comb=1, cam_scale=1.0, depth_min=-1.0, depth_max=-1.0,
                seed=20240601, device=0, images_folder="", mslp_folder="", output_folder="", synthetic=None,
                color_processing=False, import_apd=False, all_views=False, no_weak_texture=False, write_ply=False, wmf=False, no_slic=False, no_write=False, resume=False, fuse=False,
-               regions_file=None, regions_text=None, regions_size=None, lanes=2, io_threads=4, eval=None, eval_thresholds=None)
+               regions_file=None, regions_text=None, regions_size=None, lanes=2, io_threads=4, eval=None, eval_thresholds=None,
+               mesh=False, mesh_voxel=None, mesh_bbox=None, mesh_trunc=None, mesh_min_weight=None)
     i = 0
     while i < len(argv):
         a = argv[i]
@@ -283,6 +290,10 @@ def run(argv):
             _, names = write_synthetic_dataset(opt["synthetic"], mslp)
         opt["images"] = opt["images"] or names
         opt["images_folder"] = os.path.join(mslp, "images/")
+    if opt["mesh"] and int(os.environ.get("WORLD_SIZE", "1")) > 1:
+        print("[tsar_cli] -mesh runs on one GPU (every grid point reads every view): run -all_views under several ranks "
+              "without -mesh, then `tsar_cli.py -mesh -mslp_folder ...` as a single process", file=sys.stderr)
+        return 2
     if opt["all_views"]:
         if opt["fuse"] and int(os.environ.get("WORLD_SIZE", "1")) > 1:
             print("[tsar_cli] -fuse runs on one GPU (view v depends on the views before it): run -all_views under several "
@@ -295,6 +306,10 @@ def run(argv):
         run_all_views(opt, mslp)
         if opt["fuse"]:
             rc = run_fuse(opt, mslp)
+            if rc or not (opt["mesh"] or opt["eval"]):
+                return rc
+        if opt["mesh"]:
+            rc = run_mesh(opt, mslp)
             if rc or not opt["eval"]:
                 return rc
         if opt["eval"]:
@@ -302,6 +317,10 @@ def run(argv):
         return 0
     if opt["fuse"]:
         rc = run_fuse(opt, mslp)
+        if rc or not (opt["mesh"] or opt["eval"]):
+            return rc
+    if opt["mesh"]:
+        rc = run_mesh(opt, mslp)
         if rc or not opt["eval"]:
             return rc
     if opt["eval"]:
@@ -375,23 +394,53 @@ def read_pair_table(path):
     return table
 
 
+def dataset_views(opt, mslp, files):
+    """(image folder, image names as -all_views lists them, the loader of one view) of a dataset whose views all have
+    `files` under APD/<stem>/.  load(k) gives K R t from cams/ (cam_scale applied), the maps (TSAR_disp.dmb as depth,
+    TSAR_normals.dmb as normals, when listed) and the colour image (unless image=False).  Raises ValueError when there is
+    no image and FileNotFoundError naming every view whose outputs are missing."""
+    import cv2
+    folder = opt["images_folder"] or os.path.join(mslp, "images/")
+    names = opt["images"] or sorted(n for n in os.listdir(folder) if n.lower().endswith((".jpg", ".jpeg", ".png", ".npy")))
+    if not names:
+        raise ValueError(f"no images in {folder}")
+    apd = [os.path.join(mslp, "APD", n[:8]) for n in names]
+    missing = [n[:8] for n, d in zip(names, apd) if not all(os.path.exists(os.path.join(d, f)) for f in files)]
+    if missing:
+        raise FileNotFoundError(f"no {' / '.join(files)} under {os.path.join(mslp, 'APD')} for view(s) {', '.join(missing)}: "
+                                f"compute them first (-all_views)")
+
+    def load(k, image=True):
+        n = names[k]
+        K, R, t, _, _ = read_cam_txt(os.path.join(mslp, "cams", f"{n[:8]}_cam.txt"))
+        K = K.copy()
+        K[:2] /= opt["cam_scale"]
+        v = dict(K=K, R=R, t=t)
+        if image:                          # the image before the maps, the order -fuse has always read them in
+            path = os.path.join(folder, n)
+            if n.endswith(".npy"):
+                bgr = np.repeat(np.clip(np.load(path), 0, 255).astype(np.uint8)[..., None], 3, axis=-1)
+            else:
+                bgr = cv2.imread(path, cv2.IMREAD_COLOR)
+                if bgr is None:
+                    raise FileNotFoundError(path)
+            v["bgr"] = bgr
+        v["depth"] = dmb.read_dmb(os.path.join(apd[k], "TSAR_disp.dmb"))
+        if "TSAR_normals.dmb" in files:
+            v["normals"] = dmb.read_dmb(os.path.join(apd[k], "TSAR_normals.dmb"))
+        return v
+
+    return folder, names, load
+
+
 def read_fusion_views(opt, mslp, lazy=False):
     """The inputs of fusion.fuse for every image of the dataset (names as -all_views lists them): depth and normals from
     APD/<stem>/, K R t from cams/ (cam_scale applied), the colour image, and the pair.txt neighbours that exist in the
     dataset.  Raises FileNotFoundError naming every view whose outputs are missing, ValueError when there is no image or
     naming every view with no neighbour in the dataset or more than 32.  lazy=True returns (number of views, generator
     of the views) so that only one view is held in host memory at a time."""
-    import cv2
     from .fusion import MAX_NEIGHBOURS
-    folder = opt["images_folder"] or os.path.join(mslp, "images/")
-    names = opt["images"] or sorted(n for n in os.listdir(folder) if n.lower().endswith((".jpg", ".jpeg", ".png", ".npy")))
-    if not names:
-        raise ValueError(f"no images in {folder}")
-    apd = [os.path.join(mslp, "APD", n[:8]) for n in names]
-    missing = [n[:8] for n, d in zip(names, apd) if not all(os.path.exists(os.path.join(d, f)) for f in ("TSAR_disp.dmb", "TSAR_normals.dmb"))]
-    if missing:
-        raise FileNotFoundError(f"no TSAR_disp.dmb / TSAR_normals.dmb under {os.path.join(mslp, 'APD')} for view(s) {', '.join(missing)}: "
-                                f"compute them first (-all_views)")
+    _, names, load_view = dataset_views(opt, mslp, ("TSAR_disp.dmb", "TSAR_normals.dmb"))
     ids = [int(n[4:8]) for n in names]
     by_id = {c: k for k, c in enumerate(ids)}
     pairs = read_pair_table(os.path.join(mslp, "pair.txt"))
@@ -402,20 +451,7 @@ def read_fusion_views(opt, mslp, lazy=False):
                          f"view(s) {', '.join(bad)} have not")
 
     def load(k):
-        n = names[k]
-        K, R, t, _, _ = read_cam_txt(os.path.join(mslp, "cams", f"{n[:8]}_cam.txt"))
-        K = K.copy()
-        K[:2] /= opt["cam_scale"]
-        path = os.path.join(folder, n)
-        if n.endswith(".npy"):
-            bgr = np.repeat(np.clip(np.load(path), 0, 255).astype(np.uint8)[..., None], 3, axis=-1)
-        else:
-            bgr = cv2.imread(path, cv2.IMREAD_COLOR)
-            if bgr is None:
-                raise FileNotFoundError(path)
-        return dict(K=K, R=R, t=t, depth=dmb.read_dmb(os.path.join(apd[k], "TSAR_disp.dmb")),
-                    normals=dmb.read_dmb(os.path.join(apd[k], "TSAR_normals.dmb")), bgr=bgr,
-                    neighbours=neighbours[k])
+        return dict(load_view(k), neighbours=neighbours[k])
 
     if lazy:
         return len(names), (load(k) for k in range(len(names)))
@@ -443,6 +479,88 @@ def run_fuse(opt, mslp, quiet=False):
     dmb.write_fused_ply(out, xyz, nrm, rgb)
     if not quiet:
         print(f"[tsar_cli] fused {n_views} views ({W}x{H}) into {len(xyz)} points in {time.perf_counter() - t0:.2f} s -> {out}")
+    return 0
+
+
+def parse_mesh_options(opt):
+    """-mesh_voxel / -mesh_bbox / -mesh_trunc / -mesh_min_weight: (voxel or None, (lo, hi) or None, trunc or None,
+    min_weight).  Raises a one-line ValueError naming the bad option."""
+    def positive(key):
+        if opt[key] is None:
+            return None
+        try:
+            v = float(opt[key])
+        except ValueError:
+            v = math.nan
+        if not (math.isfinite(v) and v > 0 and np.float32(v) > 0 and math.isfinite(np.float32(v))):
+            raise ValueError(f"-{key}: bad value {opt[key]!r} (need a finite value > 0)")
+        return v
+    voxel, trunc = positive("mesh_voxel"), positive("mesh_trunc")
+    box = None
+    if opt["mesh_bbox"] is not None:
+        try:
+            b = [float(x) for x in opt["mesh_bbox"].split(",")]
+        except ValueError:
+            b = []
+        if len(b) != 6 or not all(math.isfinite(x) for x in b) or not all(b[a] < b[a + 3] for a in range(3)):
+            raise ValueError(f"-mesh_bbox: bad box {opt['mesh_bbox']!r} (need x0,y0,z0,x1,y1,z1, finite, with x0 < x1, "
+                             f"y0 < y1, z0 < z1)")
+        box = (b[:3], b[3:])
+    min_weight = 3
+    if opt["mesh_min_weight"] is not None:
+        try:
+            min_weight = int(opt["mesh_min_weight"])
+        except ValueError:
+            min_weight = 0
+        if not 1 <= min_weight <= 65535:
+            raise ValueError(f"-mesh_min_weight: bad value {opt['mesh_min_weight']!r} (need an integer in [1, 65535])")
+    return voxel, box, trunc, min_weight
+
+
+def mesh_grid(points, ratios, voxel, box, trunc):
+    """The grid of -mesh from the views' depth samples: the box of what they see widened by trunc (4 voxels by default),
+    or the -mesh_bbox box; the voxel is -mesh_voxel or the default voxel.  A -mesh_bbox grid never depends on the size of
+    the default box."""
+    from . import mesh
+    if box is None:
+        return mesh.grid_from_samples(points, ratios, voxel, margin=trunc)
+    return mesh.box_grid(box[0], box[1], voxel if voxel is not None else mesh.default_voxel(ratios))
+
+
+def run_mesh(opt, mslp, quiet=False):
+    """-mesh: every view's depth map and colour image -> <mslp>/TSAR_mesh.ply.  Returns the exit code."""
+    import time
+    from . import mesh
+    from .engine import TsarError
+    t0 = time.perf_counter()
+    try:
+        voxel, box, trunc, min_weight = parse_mesh_options(opt)
+        _, names, load_view = dataset_views(opt, mslp, ("TSAR_disp.dmb",))
+        # the grid first (depth maps and cams only), so that a grid that cannot be built fails before any upload
+        samples = [mesh.depth_samples(load_view(k, image=False)) for k in range(len(names))]
+        points, ratios = np.concatenate([p for p, _ in samples]), np.concatenate([r for _, r in samples])
+        grid = mesh_grid(points, ratios, voxel, box, trunc)
+        eng = None
+        try:
+            for k in range(len(names)):
+                v = load_view(k)
+                if eng is None:
+                    H, W = v["depth"].shape
+                    eng = mesh.MeshEngine(len(names), W, H, device=int(opt["device"]))
+                eng.set_view(k, v["K"], v["R"], v["t"], v["depth"], v["bgr"])
+            xyz, rgb, tri = eng.run(grid, trunc, min_weight)
+        finally:
+            if eng is not None:
+                eng.close()
+    except (FileNotFoundError, ValueError, TsarError) as e:
+        print(f"[tsar_cli] -mesh: {e}", file=sys.stderr)
+        return 1
+    out = os.path.join(mslp, "TSAR_mesh.ply")
+    dmb.write_mesh_ply(out, xyz, rgb, tri)
+    if not quiet:
+        nx, ny, nz = grid["dims"]
+        print(f"[tsar_cli] meshed {len(names)} views ({W}x{H}) on a {nx}x{ny}x{nz} grid (voxel {grid['voxel']:g}) into "
+              f"{len(xyz)} vertices and {len(tri)} triangles in {time.perf_counter() - t0:.2f} s -> {out}")
     return 0
 
 

@@ -26,6 +26,7 @@
 #include "../../include/tsar_b200.h"
 #include "dev_mem.h"
 #include "pm_math.cuh"
+#include "view_project.cuh"
 
 using namespace tsar;
 
@@ -45,12 +46,6 @@ struct ViewArgs {
     int src[TSAR_FUSION_MAX_NEIGHBOURS];
 };
 
-__device__ __forceinline__ float dot3s(float a0, float b0, float a1, float b1, float a2, float b2) {
-    return fadd(fadd(fmul(a0, b0), fmul(a1, b1)), fmul(a2, b2));
-}
-
-__device__ __forceinline__ bool valid_depth(float d) { return d > 0.0f && d <= 3.402823466e38f; }
-
 // X = R^T (d * Kinv (x, y, 1) - t)
 __device__ __forceinline__ float3 backproject(const FusionCam &c, float x, float y, float d) {
     const float rx = fadd(fadd(fmul(c.Kinv[0], x), fmul(c.Kinv[1], y)), c.Kinv[2]);
@@ -61,16 +56,6 @@ __device__ __forceinline__ float3 backproject(const FusionCam &c, float x, float
     const float cz = fsub(fmul(d, rz), c.t[2]);
     return make_float3(dot3s(c.R[0], cx, c.R[3], cy, c.R[6], cz), dot3s(c.R[1], cx, c.R[4], cy, c.R[7], cz),
                        dot3s(c.R[2], cx, c.R[5], cy, c.R[8], cz));
-}
-
-// c = R X + t, z = c.z, continuous pixel = (K c) / z
-__device__ __forceinline__ void project(const FusionCam &c, float3 X, float &px, float &py, float &z) {
-    const float cx = fadd(dot3s(c.R[0], X.x, c.R[1], X.y, c.R[2], X.z), c.t[0]);
-    const float cy = fadd(dot3s(c.R[3], X.x, c.R[4], X.y, c.R[5], X.z), c.t[1]);
-    const float cz = fadd(dot3s(c.R[6], X.x, c.R[7], X.y, c.R[8], X.z), c.t[2]);
-    z = cz;
-    px = fdiv(dot3s(c.K[0], cx, c.K[1], cy, c.K[2], cz), cz);
-    py = fdiv(dot3s(c.K[3], cx, c.K[4], cy, c.K[5], cz), cz);
 }
 
 __device__ __forceinline__ float norm3(float x, float y, float z) { return __fsqrt_rn(dot3s(x, x, y, y, z, z)); }

@@ -89,6 +89,46 @@ def read_model_ply(path):
     return rec["p"], rec["n"], rec["c"]
 
 
+MESH_VERTEX = [("p", "<f4", 3), ("c", "u1", 3)]    # float x y z, uchar red green blue
+MESH_FACE = [("n", "u1"), ("v", "<i4", 3)]          # list uchar int vertex_indices, always 3
+
+
+def write_mesh_ply(path, xyz, rgb, triangles):
+    """A triangle mesh (mesh.mesh) as binary little-endian PLY: vertex float x y z, uchar red green blue; face list uchar
+    int vertex_indices.  read_mesh_ply reads it back, read_ply_points reads its vertices."""
+    xyz = np.asarray(xyz, np.float32).reshape(-1, 3)
+    tri = np.asarray(triangles, np.int32).reshape(-1, 3)
+    vert = np.zeros(len(xyz), dtype=MESH_VERTEX)
+    vert["p"], vert["c"] = xyz, np.asarray(rgb, np.uint8).reshape(-1, 3)
+    face = np.zeros(len(tri), dtype=MESH_FACE)
+    face["n"], face["v"] = 3, tri
+    with open(path, "wb") as f:
+        f.write(("ply\nformat binary_little_endian 1.0\n" + f"element vertex {len(vert)}\n" +
+                 "property float x\nproperty float y\nproperty float z\nproperty uchar red\nproperty uchar green\n"
+                 "property uchar blue\n" + f"element face {len(face)}\n" + "property list uchar int vertex_indices\n"
+                 "end_header\n").encode())
+        vert.tofile(f)
+        face.tofile(f)
+
+
+def read_mesh_ply(path):
+    """Reader for write_mesh_ply's files: (xyz [n][3] float32, rgb [n][3] uint8, triangles [m][3] int32)."""
+    with open(path, "rb") as f:
+        counts = {}
+        while True:
+            line = f.readline().decode().strip()
+            if line.startswith("element"):
+                _, name, n = line.split()
+                counts[name] = int(n)
+            if line == "end_header":
+                break
+        vert = np.fromfile(f, dtype=MESH_VERTEX, count=counts["vertex"])
+        face = np.fromfile(f, dtype=MESH_FACE, count=counts["face"])
+    if len(vert) != counts["vertex"] or len(face) != counts["face"] or (face["n"] != 3).any():
+        raise ValueError(f"{path}: not a triangle mesh as write_mesh_ply writes it")
+    return vert["p"], vert["c"], face["v"]
+
+
 PLY_SCALARS = {"char": "i1", "int8": "i1", "uchar": "u1", "uint8": "u1", "short": "i2", "int16": "i2", "ushort": "u2",
                "uint16": "u2", "int": "i4", "int32": "i4", "uint": "u4", "uint32": "u4", "float": "f4", "float32": "f4",
                "double": "f8", "float64": "f8"}
