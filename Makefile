@@ -30,7 +30,7 @@ oracle: oracle/liboracle_cpu.so oracle/libfusion_cpu.so oracle/libeval_cpu.so or
 	bash oracle/build_ref.sh
 
 oracle/liboracle_cpu.so: oracle/oracle_cpu.c oracle/oracle_cpu.h
-	gcc -O2 -std=c11 -fPIC -shared -ffp-contract=off -fno-fast-math -o $@ oracle/oracle_cpu.c -lm
+	gcc -O2 -std=c11 -fPIC -shared -ffp-contract=off -fno-fast-math -fopenmp -o $@ oracle/oracle_cpu.c -lm
 
 oracle/libfusion_cpu.so: oracle/fusion_cpu.c include/tsar_b200.h
 	gcc -O2 -std=c11 -fPIC -shared -ffp-contract=off -fno-fast-math -o $@ oracle/fusion_cpu.c -lm

@@ -13,7 +13,7 @@ def build():
     src = os.path.join(_HERE, "oracle_cpu.c")
     if not os.path.exists(LIB) or os.path.getmtime(LIB) < max(os.path.getmtime(src), os.path.getmtime(os.path.join(_HERE, "oracle_cpu.h"))):
         subprocess.check_call(["gcc", "-O2", "-std=c11", "-fPIC", "-shared", "-ffp-contract=off", "-fno-fast-math",
-                               "-o", LIB, src, "-lm"])
+                               "-fopenmp", "-o", LIB, src, "-lm"])
     return LIB
 
 
@@ -35,6 +35,7 @@ class CpuOracle:
         L.oc_tex.restype = C.c_float
         L.oc_tex.argtypes = [vp, i, i, C.c_float, C.c_float]
         L.oc_eval_planes.argtypes = [vp, i, vp, vp, i, vp, vp, vp]
+        L.oc_eval_views.argtypes = [vp, i, vp, vp, i, vp, vp]
         L.oc_init.argtypes = [vp, C.c_uint64]
         L.oc_init_planes_only.argtypes = [vp, C.c_uint64]
         L.oc_spatial.argtypes = [vp, i]
@@ -43,6 +44,7 @@ class CpuOracle:
         L.oc_output.argtypes = [vp, vp]
         imgs = [np.ascontiguousarray(im, np.float32) for im in images]
         self.H, self.W = imgs[0].shape
+        self.V = len(subset)
         ptrs = (C.c_void_p * len(imgs))(*[im.ctypes.data for im in imgs])
         sub = (C.c_int * len(subset))(*[int(s) for s in subset])
         self.h = C.c_void_p(L.oc_create(self.W, self.H, len(imgs), ptrs, cams_struct, float(cam_f), sub, len(subset), C.byref(params)))
@@ -74,6 +76,17 @@ class CpuOracle:
         self.lib.oc_eval_planes(self.h, n, xy.ctypes.data, planes.ctypes.data, int(wrapper_rounding), cost.ctypes.data,
                                 bv.ctypes.data, ratio.ctypes.data)
         return cost, bv, ratio
+
+    def eval_views(self, xy, planes, wrapper_rounding=False):
+        """[n][V] pmCost of each selected view (subset order) for each pair, and [n][V] float64 relative variance
+        var / E[src^2] of that view's bilateral-weighted source samples."""
+        xy = np.ascontiguousarray(xy, np.int32).reshape(-1, 2)
+        planes = np.ascontiguousarray(planes, np.float32).reshape(-1, 4)
+        out = np.empty((len(xy), self.V), np.float32)
+        rel = np.empty((len(xy), self.V), np.float64)
+        self.lib.oc_eval_views(self.h, len(xy), xy.ctypes.data, planes.ctypes.data, int(wrapper_rounding), out.ctypes.data,
+                               rel.ctypes.data)
+        return out, rel
 
     def init_planes(self, seed): self.lib.oc_init(self.h, int(seed))
     def init_planes_only(self, seed): self.lib.oc_init_planes_only(self.h, int(seed))

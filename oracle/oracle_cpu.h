@@ -17,6 +17,7 @@ void oc_xorwow_row(uint64_t seed, int y, int n, uint32_t *out);
 float oc_tex(const float *img, int W, int H, float x, float y);
 float oc_multiview(oc_ctx *c, int x, int y, const float *pl, int hrad, int vrad, int pxf, int *beview, float *ratio);
 void oc_eval_planes(oc_ctx *c, int n, const int *xy, const float *planes, int pxf, float *cost, int *beview, float *ratio);
+void oc_eval_views(oc_ctx *c, int n, const int *xy, const float *planes, int pxf, float *cost, double *src_rel);
 void oc_init(oc_ctx *c, uint64_t seed);
 void oc_init_planes_only(oc_ctx *c, uint64_t seed);
 void oc_spatial(oc_ctx *c, int colour);
